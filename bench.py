@@ -52,7 +52,47 @@ def parse():
                     "pipelining across launches, see HipsCNNTrainStep(lookahead=...)); measured: no gain at 1-2 GPUs, so not the default")
     ap.add_argument("--fast", action="store_true", help="plain TF32 tensor-core products instead of the fp32-accurate 3xTF32 default")
     ap.add_argument("--wire-dtype", default="fp32", choices=["fp32", "fp16", "mpq", "fp8"], help="transport format of the fused HiPS step (FP16 / MPQ accelerators)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last timed step computed on rank 0 (per-sample "
+                    "loss, logits where the engine keeps them, the updated parameters) as DIR/<name>.npy in float32, so that two builds run with "
+                    "the same arguments can be compared output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def step_outputs(eng):
+    """The arrays a caller of ``eng.run_device()`` receives from the step just run: per-sample loss, logits (fused engine only) and the
+    updated parameters in ``CNN_PARAM_SHAPES`` order."""
+    if isinstance(eng, ScriptPathEngine):
+        out = {"loss": eng._loss._t}
+        params = [p.data()._t for p in eng.params]
+    else:
+        out = {"loss": eng.loss}
+        if getattr(eng, "logits", None) is not None:
+            out["logits"] = eng.logits
+        params = eng.P
+    for i, p in enumerate(params):
+        out["param_%02d" % i] = p
+    return out
+
+
+def dump_outputs(arrays, out_dir):
+    """Write ``arrays`` as float32 ``.npy`` files.  If they exceed ``DUMP_LIMIT_BYTES`` together, every array larger than an equal share of
+    the limit is replaced by a fixed, seeded sample of its flattened elements (same indices on every run)."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    host = {k: v.detach().float().cpu().numpy() for k, v in arrays.items()}
+    share = DUMP_LIMIT_BYTES // 4 // len(host)
+    sample = sum(a.size for a in host.values()) * 4 > DUMP_LIMIT_BYTES
+    for name, a in host.items():
+        if sample and a.size > share:
+            idx = np.sort(np.random.default_rng(0).choice(a.size, share, replace=False))
+            a = a.reshape(-1)[idx]
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a, dtype=np.float32))
 
 
 class ClockSampler:
@@ -252,6 +292,8 @@ def main():
         eng.run_device()
         ends[i].record()
     barrier()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(step_outputs(eng), args.dump_outputs)      # before the e2e region below trains on
     per_step = sorted(s.elapsed_time(e) for s, e in zip(starts, ends))
     dev_ms = sum(per_step)
     pct = lambda q: per_step[min(K - 1, int(q * K))]

@@ -33,3 +33,7 @@ for step in range(int(os.environ.get("TEST_STEPS", "2"))):
 kv._barrier()
 with open(os.path.join(os.environ["TEST_OUT_DIR"], "rank%d.json" % rank), "w") as f:      # ranks share one stdout: lines may interleave
     json.dump(out, f)
+# tear the gloo process group down before interpreter shutdown: left to exit-time destruction it can abort the process
+# ("terminate called without an active exception") and fail the launch
+import torch.distributed as dist  # noqa: E402
+dist.destroy_process_group()
