@@ -13,7 +13,13 @@
 
 #define GX_CAPI extern "C" __attribute__((visibility("default")))
 
+namespace gxrt { namespace capi { bool IsDeviceBuffer(const void* p); } }    // runtime/c_api_runtime.cc
+
 namespace {
+// buffers of device NDArrays (GXNDArrayGetData) are refused: the parameter-server plane reads and writes host memory
+void HostOnly(const void* p, const char* fn) {
+  if (p && gxrt::capi::IsDeviceBuffer(p)) throw std::runtime_error(std::string(fn) + ": device array (the KVStore group works on host buffers only)");
+}
 thread_local std::string last_error;
 template <typename F>
 int Guard(F&& f) {
@@ -46,18 +52,18 @@ GX_CAPI int GXKVStoreGetNumAllWorkers(void* h, int* out) { return Guard([&] { *o
 GX_CAPI int GXKVStoreIsMasterWorker(void* h, int* out) { return Guard([&] { *out = KV(h)->is_master_worker(); }); }
 
 // dtype: mshadow flags (0 f32, 1 f64, 2 f16, 3 u8, 4 i32, 5 i8, 6 i64, 12 bf16).  The caller keeps `data` alive until the handle was waited.
-GX_CAPI int GXKVStoreInit(void* h, int key, const void* data, size_t elems, int dtype) { return Guard([&] { KV(h)->Init(key, data, elems, dtype); }); }
+GX_CAPI int GXKVStoreInit(void* h, int key, const void* data, size_t elems, int dtype) { return Guard([&] { HostOnly(data, "GXKVStoreInit"); KV(h)->Init(key, data, elems, dtype); }); }
 GX_CAPI int GXKVStorePush(void* h, int key, const void* data, size_t elems, int dtype, int priority, int* handle) {
-  return Guard([&] { const int r = KV(h)->Push(key, data, elems, dtype, priority); if (handle) *handle = r; });
+  return Guard([&] { HostOnly(data, "GXKVStorePush"); const int r = KV(h)->Push(key, data, elems, dtype, priority); if (handle) *handle = r; });
 }
 GX_CAPI int GXKVStorePull(void* h, int key, void* out, size_t elems, int dtype, int priority, int* handle) {
-  return Guard([&] { const int r = KV(h)->Pull(key, out, elems, dtype, priority); if (handle) *handle = r; });
+  return Guard([&] { HostOnly(out, "GXKVStorePull"); const int r = KV(h)->Pull(key, out, elems, dtype, priority); if (handle) *handle = r; });
 }
 GX_CAPI int GXKVStorePushRowSparse(void* h, int key, const int64_t* row_ids, size_t nrows, const float* rows, size_t row_len, int priority, int* handle) {
-  return Guard([&] { const int r = KV(h)->PushRows(key, row_ids, nrows, rows, row_len, priority); if (handle) *handle = r; });
+  return Guard([&] { HostOnly(rows, "GXKVStorePushRowSparse"); const int r = KV(h)->PushRows(key, row_ids, nrows, rows, row_len, priority); if (handle) *handle = r; });
 }
 GX_CAPI int GXKVStorePullRowSparse(void* h, int key, const int64_t* row_ids, size_t nrows, float* out, size_t row_len, int priority, int* handle) {
-  return Guard([&] { const int r = KV(h)->PullRows(key, row_ids, nrows, out, row_len, priority); if (handle) *handle = r; });
+  return Guard([&] { HostOnly(out, "GXKVStorePullRowSparse"); const int r = KV(h)->PullRows(key, row_ids, nrows, out, row_len, priority); if (handle) *handle = r; });
 }
 GX_CAPI int GXKVStoreWait(void* h, int handle) { return Guard([&] { KV(h)->Wait(handle); }); }
 GX_CAPI int GXKVStoreWaitAll(void* h) { return Guard([&] { KV(h)->WaitAll(); }); }

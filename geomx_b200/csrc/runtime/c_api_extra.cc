@@ -2,7 +2,8 @@
 //
 // Parity: include/mxnet/c_api.h
 //   :560-760    MXNDArrayCreateNone / Slice / At / Reshape / GetContext / GetStorageType / WaitToRead / WaitToWrite / WaitAll /
-//               SaveRawBytes / LoadFromRawBytes   (host arrays are synchronous, so the wait functions only order against the C engine)
+//               SaveRawBytes / LoadFromRawBytes   (host arrays are synchronous; for device arrays the wait functions synchronise the
+//               library stream of the array's device, WaitAll every device stream and the C engine)
 //   :280-420    MXProfileCreateDomain / CreateTask / CreateFrame / CreateEvent / CreateCounter / DestroyHandle / DurationStart / DurationStop /
 //               SetCounter / AdjustCounter        (src/c_api/c_api_profile.cc:300-560)
 //   :190-260    MXSetNumOMPThreads / MXEngineSetBulkSize / MXGetGPUCount / MXNotifyShutdown
@@ -59,23 +60,25 @@ GX_CAPI int GXNDArrayCreateNone(void** out) { return Guard([&] { *out = new Host
 GX_CAPI int GXNDArraySlice(void* h, uint32_t begin, uint32_t end, void** out) {
   return Guard([&] {
     HostArray* a = ND(h);
+    const std::string& data = gxrt::capi::HostBytes(a, "GXNDArraySlice");
     if (a->rec.shape.empty() || begin > end || end > static_cast<uint32_t>(a->rec.shape[0])) throw std::runtime_error("Slice: range out of bounds");
-    const size_t row = a->rec.data.size() / static_cast<size_t>(std::max<int64_t>(a->rec.shape[0], 1));
+    const size_t row = data.size() / static_cast<size_t>(std::max<int64_t>(a->rec.shape[0], 1));
     auto s = std::make_unique<HostArray>();
     s->rec.dtype = a->rec.dtype; s->rec.shape = a->rec.shape; s->rec.shape[0] = end - begin;
-    s->rec.data.assign(a->rec.data.data() + begin * row, (end - begin) * row);
+    s->rec.data.assign(data.data() + begin * row, (end - begin) * row);
     *out = s.release();
   });
 }
 GX_CAPI int GXNDArrayAt(void* h, uint32_t idx, void** out) {
   return Guard([&] {
     HostArray* a = ND(h);
+    const std::string& data = gxrt::capi::HostBytes(a, "GXNDArrayAt");
     if (a->rec.shape.empty() || idx >= static_cast<uint32_t>(a->rec.shape[0])) throw std::runtime_error("At: index out of bounds");
-    const size_t row = a->rec.data.size() / static_cast<size_t>(a->rec.shape[0]);
+    const size_t row = data.size() / static_cast<size_t>(a->rec.shape[0]);
     auto s = std::make_unique<HostArray>();
     s->rec.dtype = a->rec.dtype; s->rec.shape.assign(a->rec.shape.begin() + 1, a->rec.shape.end());
     if (s->rec.shape.empty()) s->rec.shape.push_back(1);
-    s->rec.data.assign(a->rec.data.data() + idx * row, row);
+    s->rec.data.assign(data.data() + idx * row, row);
     *out = s.release();
   });
 }
@@ -83,6 +86,7 @@ GX_CAPI int GXNDArrayAt(void* h, uint32_t idx, void** out) {
 GX_CAPI int GXNDArrayReshape(void* h, int ndim, const int* dims, void** out) {
   return Guard([&] {
     HostArray* a = ND(h);
+    const std::string& data = gxrt::capi::HostBytes(a, "GXNDArrayReshape");
     const int64_t total = gxrt::Prod(a->rec.shape);
     std::vector<int64_t> shp; int infer = -1; int64_t known = 1;
     for (int i = 0; i < ndim; ++i) {
@@ -95,19 +99,25 @@ GX_CAPI int GXNDArrayReshape(void* h, int ndim, const int* dims, void** out) {
     if (infer >= 0) { if (known == 0 || total % known) throw std::runtime_error("Reshape: cannot infer -1"); shp[infer] = total / known; known *= shp[infer]; }
     if (known != total) throw std::runtime_error("Reshape: size changes from " + std::to_string(total) + " to " + std::to_string(known));
     auto s = std::make_unique<HostArray>();
-    s->rec.dtype = a->rec.dtype; s->rec.shape = shp; s->rec.data = a->rec.data;
+    s->rec.dtype = a->rec.dtype; s->rec.shape = shp; s->rec.data = data;
     *out = s.release();
   });
 }
-GX_CAPI int GXNDArrayGetContext(void* h, int* out_dev_type, int* out_dev_id) { return Guard([&] { ND(h); *out_dev_type = 1; *out_dev_id = 0; }); }   // kCPU
+// (1, 0) kCPU for host arrays, (2, dev_id) kGPU for device arrays
+GX_CAPI int GXNDArrayGetContext(void* h, int* out_dev_type, int* out_dev_id) {
+  return Guard([&] { HostArray* a = ND(h); *out_dev_type = a->device() ? 2 : 1; *out_dev_id = a->device() ? a->dev_id : 0; });
+}
 GX_CAPI int GXNDArrayGetStorageType(void* h, int* out) { return Guard([&] { *out = ND(h)->rec.shape.empty() ? -1 : 0; }); }                           // kDefaultStorage
-GX_CAPI int GXNDArrayWaitToRead(void* h) { return Guard([&] { ND(h); }); }
-GX_CAPI int GXNDArrayWaitToWrite(void* h) { return Guard([&] { ND(h); }); }
-GX_CAPI int GXNDArrayWaitAll() { return GXEngineWaitAll(); }
+GX_CAPI int GXNDArrayWaitToRead(void* h) { return Guard([&] { HostArray* a = ND(h); if (a->device()) gxrt::capi::SyncDevice(a->dev_id); }); }
+GX_CAPI int GXNDArrayWaitToWrite(void* h) { return Guard([&] { HostArray* a = ND(h); if (a->device()) gxrt::capi::SyncDevice(a->dev_id); }); }
+GX_CAPI int GXNDArrayWaitAll() {
+  if (Guard([&] { gxrt::capi::SyncAllDevices(); }) != 0) return -1;
+  return GXEngineWaitAll();
+}
 // one array in NDArray::Save's layout (src/ndarray/ndarray.cc:1583-1660); the buffer is thread-local
 GX_CAPI int GXNDArraySaveRawBytes(void* h, size_t* out_size, const char** out_buf) {
   return Guard([&] {
-    const std::string list = gxrt::WriteList({ND(h)->rec}, {});
+    const std::string list = gxrt::WriteList({gxrt::capi::HostCopy(ND(h))}, {});
     raw_bytes = list.substr(24, list.size() - 24 - 8);          // strip the list header (magic, reserved, count) and the empty name table
     *out_size = raw_bytes.size(); *out_buf = raw_bytes.data();
   });

@@ -19,6 +19,7 @@
 #include <string>
 #include <vector>
 
+#include "device_exec.h"
 #include "graph.h"
 #include "host_array.h"
 #include "train_exec.h"
@@ -47,7 +48,10 @@ struct AGNode {
   bool released = false;
 };
 
-HostArray::~HostArray() { if (ag && ag->var == this) ag->var = nullptr; }
+HostArray::~HostArray() {
+  if (ag && ag->var == this) ag->var = nullptr;
+  try { ReleaseDevice(this); } catch (...) {}
+}
 
 }  // namespace capi
 }  // namespace gxrt
@@ -92,8 +96,9 @@ struct ShapeRet {
 thread_local ShapeRet ret_shape;
 
 float* F32(HostArray* a, const char* what) {
+  std::string& bytes = gxrt::capi::HostBytes(a, what);
   if (a->rec.dtype != 0) throw std::runtime_error(std::string(what) + ": the native executor computes in float32 (dtype flag 0), got dtype flag " + std::to_string(a->rec.dtype));
-  return reinterpret_cast<float*>(&a->rec.data[0]);
+  return reinterpret_cast<float*>(&bytes[0]);
 }
 Shape ShapeOf(const HostArray* a) { return Shape(a->rec.shape.begin(), a->rec.shape.end()); }
 HostArray* NewArray(const Shape& s) {
@@ -112,6 +117,7 @@ AttrMap Attrs(uint32_t n, const char** keys, const char** vals) {
 // ---- executor handle: the executor + the arrays it hands out
 struct ExecHandle {
   std::unique_ptr<E::Executor> ex;
+  std::unique_ptr<E::DeviceExecutor> dex;                // set instead of ex for graphs bound to device arrays; outputs are views of its memory
   std::vector<std::unique_ptr<HostArray>> outputs;
   std::vector<std::unique_ptr<HostArray>> owned;        // SimpleBind: arguments / gradients / auxiliary states allocated here
   std::string printed;
@@ -131,6 +137,38 @@ ExecHandle* BindImpl(Symbol* sym, const std::vector<HostArray*>& args, const std
   h->ex.reset(new E::Executor(*sym, ta, tg, reqs, tx));
   for (size_t i = 0; i < h->ex->NumOutputs(); ++i) h->outputs.emplace_back(NewArray(h->ex->OutputShape(i)));
   return h.release();
+}
+// all arrays on device dev: the device executor; outputs are device arrays that view the executor's output buffers
+ExecHandle* BindDeviceImpl(Symbol* sym, int dev, const std::vector<HostArray*>& args, const std::vector<HostArray*>& grads, const std::vector<int>& reqs,
+                           const std::vector<HostArray*>& aux) {
+  std::vector<E::Tensor> ta, tg, tx;
+  for (auto* a : args) ta.push_back({a->dptr, ShapeOf(a)});
+  for (size_t i = 0; i < args.size(); ++i) {
+    HostArray* g = i < grads.size() ? grads[i] : nullptr;
+    if (g && i < reqs.size() && reqs[i] != E::kNullOp) tg.push_back({g->dptr, ShapeOf(g)}); else tg.push_back({nullptr, {}});
+  }
+  for (auto* a : aux) tx.push_back({a->dptr, ShapeOf(a)});
+  auto h = std::make_unique<ExecHandle>();
+  h->dex.reset(new E::DeviceExecutor(*sym, dev, ta, tg, reqs, tx));
+  for (size_t i = 0; i < h->dex->NumOutputs(); ++i) {
+    auto o = std::make_unique<HostArray>();
+    const Shape& s = h->dex->OutputShape(i);
+    o->rec.dtype = 0; o->rec.shape.assign(s.begin(), s.end()); o->dev_id = dev; o->dptr = h->dex->OutputData(i); o->owns_dptr = false;
+    h->outputs.push_back(std::move(o));
+  }
+  return h.release();
+}
+// where the arrays of a bind live: -1 all on the host, d >= 0 all on device d; a mix or several devices is an error
+int BindDevice(const char* fn, const std::vector<HostArray*>& arrays) {
+  int dev = -2;
+  for (HostArray* a : arrays) {
+    if (!a) continue;
+    const int d = a->device() ? a->dev_id : -1;
+    if (dev == -2) dev = d;
+    else if (d != dev) throw std::runtime_error(std::string(fn) + ": arrays on " + (dev < 0 ? std::string("the host") : "gpu(" + std::to_string(dev) + ")") + " and " +
+                                                (d < 0 ? std::string("the host") : "gpu(" + std::to_string(d) + ")") + " cannot be bound together");
+  }
+  return dev == -2 ? -1 : dev;
 }
 void PublishOutputs(ExecHandle* h) {
   for (size_t i = 0; i < h->outputs.size(); ++i) memcpy(&h->outputs[i]->rec.data[0], h->ex->OutputData(i), h->outputs[i]->rec.data.size());
@@ -157,14 +195,15 @@ void BackwardImpl(uint32_t num, void** outs, void** ograds, bool retain) {
   };
   for (uint32_t i = 0; i < num; ++i) {
     HostArray* o = ND(outs[i]);
+    if (o->device()) throw std::runtime_error("GXAutogradBackward: device array (autograd records host arrays only)");
     if (!o->ag) throw std::runtime_error("Backward: output " + std::to_string(i) + " was not computed while recording (or its graph was already freed)");
     CollectTopo(o->ag, &seen, &order);
     const size_t n = o->rec.data.size() / 4;
     auto& g = slot(o->ag.get(), o->ag_out, n);
     if (ograds && ograds[i]) {
       HostArray* og = ND(ograds[i]);
+      const float* p = F32(og, "GXAutogradBackward");
       if (og->rec.data.size() != o->rec.data.size()) throw std::runtime_error("Backward: head gradient " + std::to_string(i) + " does not match its output");
-      const float* p = F32(og, "head gradient");
       for (size_t k = 0; k < n; ++k) g[k] += p[k];
     } else for (auto& v : g) v += 1.f;
   }
@@ -418,11 +457,11 @@ GX_CAPI int GXSymbolInferType(void* sym, uint32_t num_args, const char** keys, c
 }
 
 // ================================================================================================ Executor
-// dev_type / dev_id are accepted for signature parity: this executor runs on the host (device execution = the Python Executor / CUDA graphs).
+// Host arrays bind the host executor (dev_type / dev_id are then accepted for signature parity only).  Device arrays, all on gpu(dev_id) with
+// dev_type 2, bind the device executor (device_exec.h); mixing host and device arrays, or devices, is an error.
 // grad_req_type: 0 null, 1 write, 3 add (include/mxnet/op_attr_types.h OpReqType).
 GX_CAPI int GXExecutorBind(void* sym, int dev_type, int dev_id, uint32_t len, void** in_args, void** arg_grad_store, const uint32_t* grad_req_type,
                            uint32_t aux_states_len, void** aux_states, void** out) {
-  (void)dev_type; (void)dev_id;
   return Guard([&] {
     std::vector<HostArray*> args, grads, aux; std::vector<int> reqs;
     for (uint32_t i = 0; i < len; ++i) {
@@ -431,16 +470,27 @@ GX_CAPI int GXExecutorBind(void* sym, int dev_type, int dev_id, uint32_t len, vo
       reqs.push_back(grad_req_type && grads.back() ? static_cast<int>(grad_req_type[i]) : E::kNullOp);
     }
     for (uint32_t i = 0; i < aux_states_len; ++i) aux.push_back(ND(aux_states[i]));
-    *out = BindImpl(SYM(sym), args, grads, reqs, aux);
+    std::vector<HostArray*> all = args;
+    all.insert(all.end(), grads.begin(), grads.end()); all.insert(all.end(), aux.begin(), aux.end());
+    const int dev = BindDevice("GXExecutorBind", all);
+    if (dev < 0) { *out = BindImpl(SYM(sym), args, grads, reqs, aux); return; }
+    if (dev_type != 2 || dev_id != dev)
+      throw std::runtime_error("GXExecutorBind: the arrays live on gpu(" + std::to_string(dev) + "), the bind asks for dev_type " + std::to_string(dev_type) + " dev_id " + std::to_string(dev_id));
+    *out = BindDeviceImpl(SYM(sym), dev, args, grads, reqs, aux);
   });
 }
 // Allocates every argument, gradient and auxiliary array from the given input shapes (role of MXExecutorSimpleBind, c_api.h:1640; the
 // signature is reduced to what a host executor needs).  grad_req: "null" | "write" | "add" for all arguments except those named in
 // `no_grad_keys` (typically data and label).  The arrays come back in ListArguments / ListAuxiliaryStates order and belong to the executor.
-GX_CAPI int GXExecutorSimpleBind(void* sym, uint32_t num_shapes, const char** keys, const uint32_t* ind_ptr, const uint32_t* shape_data, const char* grad_req,
-                                 uint32_t num_no_grad, const char** no_grad_keys, void** out, uint32_t* num_args, void*** in_args, void*** arg_grads,
-                                 uint32_t* num_aux, void*** aux_states) {
+// dev_type 1: host arrays and the host executor (GXExecutorSimpleBind).  dev_type 2: zero-filled device arrays on gpu(dev_id) and the device
+// executor.  The device's position follows the reference's MXExecutorSimpleBind (c_api.h:1640).
+GX_CAPI int GXExecutorSimpleBindEx(void* sym, int dev_type, int dev_id, uint32_t num_shapes, const char** keys, const uint32_t* ind_ptr, const uint32_t* shape_data,
+                                   const char* grad_req, uint32_t num_no_grad, const char** no_grad_keys, void** out, uint32_t* num_args, void*** in_args,
+                                   void*** arg_grads, uint32_t* num_aux, void*** aux_states) {
   return Guard([&] {
+    if (dev_type != 1 && dev_type != 2) throw std::runtime_error("GXExecutorSimpleBindEx: dev_type " + std::to_string(dev_type) + " is not supported (1 CPU, 2 GPU)");
+    const bool on_dev = dev_type == 2;
+    auto make = [&](const Shape& sh) { return on_dev ? gxrt::capi::NewDeviceArray(std::vector<int64_t>(sh.begin(), sh.end()), dev_id) : NewArray(sh); };
     Symbol* s = SYM(sym);
     std::map<std::string, Shape> known;
     for (uint32_t i = 0; i < num_shapes; ++i) known[keys[i]] = Shape(shape_data + ind_ptr[i], shape_data + ind_ptr[i + 1]);
@@ -455,13 +505,13 @@ GX_CAPI int GXExecutorSimpleBind(void* sym, uint32_t num_shapes, const char** ke
     std::vector<std::unique_ptr<HostArray>> owned;
     std::vector<HostArray*> args, grads, aux; std::vector<int> reqs;
     for (auto& n : G::ListArguments(*s)) {
-      owned.emplace_back(NewArray(by_name.at(n))); args.push_back(owned.back().get());
+      owned.emplace_back(make(by_name.at(n))); args.push_back(owned.back().get());
       const int q = no_grad.count(n) ? E::kNullOp : rq;
       reqs.push_back(q);
-      if (q != E::kNullOp) { owned.emplace_back(NewArray(by_name.at(n))); grads.push_back(owned.back().get()); } else grads.push_back(nullptr);
+      if (q != E::kNullOp) { owned.emplace_back(make(by_name.at(n))); grads.push_back(owned.back().get()); } else grads.push_back(nullptr);
     }
-    for (auto& n : G::ListAuxiliaryStates(*s)) { owned.emplace_back(NewArray(by_name.at(n))); aux.push_back(owned.back().get()); }
-    ExecHandle* h = BindImpl(s, args, grads, reqs, aux);
+    for (auto& n : G::ListAuxiliaryStates(*s)) { owned.emplace_back(make(by_name.at(n))); aux.push_back(owned.back().get()); }
+    ExecHandle* h = on_dev ? BindDeviceImpl(s, dev_id, args, grads, reqs, aux) : BindImpl(s, args, grads, reqs, aux);
     h->owned = std::move(owned);
     static thread_local std::vector<void*> ra, rg, rx;
     ra.assign(args.begin(), args.end()); rg.assign(grads.begin(), grads.end()); rx.assign(aux.begin(), aux.end());
@@ -469,7 +519,19 @@ GX_CAPI int GXExecutorSimpleBind(void* sym, uint32_t num_shapes, const char** ke
     *num_aux = static_cast<uint32_t>(rx.size()); *aux_states = rx.data();
   });
 }
-GX_CAPI int GXExecutorForward(void* h, int is_train) { return Guard([&] { ExecHandle* e = EX(h); e->ex->Forward(is_train != 0); PublishOutputs(e); }); }
+GX_CAPI int GXExecutorSimpleBind(void* sym, uint32_t num_shapes, const char** keys, const uint32_t* ind_ptr, const uint32_t* shape_data, const char* grad_req,
+                                 uint32_t num_no_grad, const char** no_grad_keys, void** out, uint32_t* num_args, void*** in_args, void*** arg_grads,
+                                 uint32_t* num_aux, void*** aux_states) {
+  return GXExecutorSimpleBindEx(sym, 1, 0, num_shapes, keys, ind_ptr, shape_data, grad_req, num_no_grad, no_grad_keys, out, num_args, in_args, arg_grads, num_aux,
+                                aux_states);
+}
+GX_CAPI int GXExecutorForward(void* h, int is_train) {
+  return Guard([&] {
+    ExecHandle* e = EX(h);
+    if (e->dex) { e->dex->Forward(is_train != 0); return; }
+    e->ex->Forward(is_train != 0); PublishOutputs(e);
+  });
+}
 // head_grads may be null / len 0 for loss heads
 GX_CAPI int GXExecutorBackward(void* h, uint32_t len, void** head_grads) {
   return Guard([&] {
@@ -478,10 +540,16 @@ GX_CAPI int GXExecutorBackward(void* h, uint32_t len, void** head_grads) {
     for (uint32_t i = 0; i < len; ++i) {
       if (!head_grads || !head_grads[i]) { hg.push_back(nullptr); continue; }
       HostArray* g = ND(head_grads[i]);
+      if (e->dex) {
+        if (!g->device() || g->dev_id != e->dex->device()) throw std::runtime_error("GXExecutorBackward: head gradient " + std::to_string(i) + " must be a device array on gpu(" + std::to_string(e->dex->device()) + ")");
+        if (i < e->outputs.size() && g->Bytes() != e->outputs[i]->Bytes()) throw std::runtime_error("Backward: head gradient " + std::to_string(i) + " does not match its output");
+        hg.push_back(g->dptr);
+        continue;
+      }
       if (i < e->outputs.size() && g->rec.data.size() != e->outputs[i]->rec.data.size()) throw std::runtime_error("Backward: head gradient " + std::to_string(i) + " does not match its output");
-      hg.push_back(F32(g, "head gradient"));
+      hg.push_back(F32(g, "GXExecutorBackward"));
     }
-    e->ex->Backward(hg);
+    if (e->dex) e->dex->Backward(hg); else e->ex->Backward(hg);
   });
 }
 GX_CAPI int GXExecutorBackwardEx(void* h, uint32_t len, void** head_grads, int is_train) { (void)is_train; return GXExecutorBackward(h, len, head_grads); }
@@ -494,7 +562,9 @@ GX_CAPI int GXExecutorOutputs(void* h, uint32_t* out_size, void*** out) {
     *out_size = static_cast<uint32_t>(r.size()); *out = r.data();
   });
 }
-GX_CAPI int GXExecutorPrint(void* h, const char** out_str) { return Guard([&] { ExecHandle* e = EX(h); e->printed = e->ex->Print(); *out_str = e->printed.c_str(); }); }
+GX_CAPI int GXExecutorPrint(void* h, const char** out_str) {
+  return Guard([&] { ExecHandle* e = EX(h); e->printed = e->dex ? e->dex->Print() : e->ex->Print(); *out_str = e->printed.c_str(); });
+}
 GX_CAPI int GXExecutorFree(void* h) { return Guard([&] { delete EX(h); }); }
 
 // ================================================================================================ imperative invoke + autograd
@@ -506,7 +576,7 @@ GX_CAPI int GXAutogradMarkVariables(uint32_t num_var, void** var_handles, const 
   return Guard([&] {
     for (uint32_t i = 0; i < num_var; ++i) {
       HostArray* v = ND(var_handles[i]); HostArray* g = ND(grad_handles[i]);
-      F32(v, "MarkVariables"); F32(g, "MarkVariables gradient");
+      F32(v, "GXAutogradMarkVariables"); F32(g, "GXAutogradMarkVariables");
       if (g->rec.data.size() != v->rec.data.size()) throw std::runtime_error("MarkVariables: gradient " + std::to_string(i) + " does not match its variable");
       v->ag = std::make_shared<AGNode>(); v->ag->var = v;
       v->grad = g; v->grad_req = static_cast<int>(reqs_array[i]);
@@ -516,10 +586,61 @@ GX_CAPI int GXAutogradMarkVariables(uint32_t num_var, void** var_handles, const 
 GX_CAPI int GXNDArrayGetGrad(void* handle, void** out) { return Guard([&] { *out = ND(handle)->grad; }); }
 // a new handle with the same contents and no history
 GX_CAPI int GXNDArrayDetach(void* handle, void** out) {
-  return Guard([&] { HostArray* a = ND(handle); auto c = std::make_unique<HostArray>(); c->rec = a->rec; *out = c.release(); });
+  return Guard([&] {
+    HostArray* a = ND(handle);
+    auto c = std::make_unique<HostArray>();
+    c->rec.dtype = a->rec.dtype; c->rec.shape = a->rec.shape; c->rec.data = gxrt::capi::HostBytes(a, "GXNDArrayDetach");
+    *out = c.release();
+  });
 }
 
-// One operator on host arrays.  *num_outputs == 0 (or *outputs == nullptr): the output array is created and returned through thread-local
+// One operator on device arrays through a one-node device executor, on the library stream of their device.  Trailing auxiliary inputs
+// (BatchNorm's running statistics, optimizer states) are bound in place; given output arrays may alias an input, since the result is copied
+// out of the executor's own buffers.
+void InvokeDevice(const OpDef* d, const Symbol& sym, int num_inputs, void** inputs, int* num_outputs, void*** outputs) {
+  std::vector<HostArray*> in;
+  for (int i = 0; i < num_inputs; ++i) in.push_back(ND(inputs[i]));
+  const int dev = BindDevice("GXImperativeInvoke", in);
+  const int n_arg = num_inputs - d->num_aux;
+  std::vector<E::Tensor> ta, tg, tx; std::vector<int> reqs;
+  for (int i = 0; i < num_inputs; ++i) {
+    if (in[i]->rec.dtype != 0) throw std::runtime_error("GXImperativeInvoke: device arrays are float32");
+    (i < n_arg ? ta : tx).push_back({in[i]->dptr, ShapeOf(in[i])});
+    if (i < n_arg) { tg.push_back({nullptr, {}}); reqs.push_back(E::kNullOp); }
+  }
+  E::DeviceExecutor ex(sym, dev, ta, tg, reqs, tx);
+  ex.Forward(ag_training);
+  const int nout = static_cast<int>(ex.NumOutputs());
+  const bool given = *num_outputs > 0 && outputs && *outputs;
+  if (given && *num_outputs != nout) throw std::runtime_error(std::string(d->name) + ": " + std::to_string(*num_outputs) + " output arrays given, the operator produces " + std::to_string(nout));
+  std::vector<HostArray*> outs;
+  for (int o = 0; o < nout; ++o) {
+    const Shape& os = ex.OutputShape(o);
+    const std::vector<int64_t> shp(os.begin(), os.end());
+    HostArray* out = nullptr;
+    if (given) {
+      out = ND((*outputs)[o]);
+      if (!out->device() || out->dev_id != dev) throw std::runtime_error("GXImperativeInvoke: output " + std::to_string(o) + " must be a device array on gpu(" + std::to_string(dev) + ")");
+      if (out->rec.shape != shp || !out->owns_dptr) {
+        std::unique_ptr<HostArray> fresh(gxrt::capi::NewDeviceArray(shp, dev));
+        gxrt::capi::ReleaseDevice(out);
+        out->dptr = fresh->dptr; out->owns_dptr = true; out->rec.shape = shp; out->rec.dtype = 0;
+        fresh->owns_dptr = false;
+      }
+    } else {
+      out = gxrt::capi::NewDeviceArray(shp, dev);
+    }
+    outs.push_back(out);
+  }
+  for (int o = 0; o < nout; ++o) {
+    const gxrt::kern::Lib& L = gxrt::kern::Get();
+    gxrt::kern::Check(L.memcpy(outs[o]->dptr, ex.OutputData(o), outs[o]->Bytes(), 3, L.stream(dev)), "GXImperativeInvoke");
+  }
+  if (!given) { ret_inv.handles.assign(outs.begin(), outs.end()); *outputs = ret_inv.handles.data(); }
+  *num_outputs = nout;
+}
+
+// One operator on host arrays (device arrays: InvokeDevice).  *num_outputs == 0 (or *outputs == nullptr): the output array is created and returned through thread-local
 // storage (the caller owns the handle, GXNDArrayFree); otherwise the given array is overwritten (resized when necessary).  While recording,
 // the invocation is kept — with a snapshot of its inputs and its forward state — so GXAutogradBackward can differentiate through it.
 GX_CAPI int GXImperativeInvoke(void* creator, int num_inputs, void** inputs, int* num_outputs, void*** outputs, int num_params, const char** param_keys,
@@ -535,6 +656,13 @@ GX_CAPI int GXImperativeInvoke(void* creator, int num_inputs, void** inputs, int
     std::vector<Symbol> vars;
     for (int i = 0; i < num_inputs; ++i) vars.push_back(G::Variable("in" + std::to_string(i)));
     G::Compose(&sym, "op", vars, {});
+    bool on_device = false;
+    for (int i = 0; i < num_inputs; ++i) on_device = on_device || ND(inputs[i])->device();
+    if (on_device) {
+      if (ag_recording) throw std::runtime_error("GXImperativeInvoke: device inputs while autograd is recording (autograd records host arrays only)");
+      InvokeDevice(d, sym, num_inputs, inputs, num_outputs, outputs);
+      return;
+    }
     auto node = std::make_shared<AGNode>();
     node->sym = sym; node->op = d->name; node->attrs = attrs;
     const int n_aux = d->num_aux, n_arg = num_inputs - n_aux;
@@ -542,7 +670,7 @@ GX_CAPI int GXImperativeInvoke(void* creator, int num_inputs, void** inputs, int
     std::vector<HostArray*> in;
     for (int i = 0; i < num_inputs; ++i) {
       HostArray* a = ND(inputs[i]);
-      const float* p = F32(a, d->name);
+      const float* p = F32(a, "GXImperativeInvoke");
       in.push_back(a);
       node->in_copy.emplace_back(p, p + a->rec.data.size() / 4);
       node->in_node.push_back(i < n_arg && ag_recording ? a->ag : nullptr);

@@ -6,11 +6,15 @@
 //   Profiler  MXSetProfilerConfig / MXSetProfilerState / MXDumpProfile / MXProfilePause / MXProfileSetMarker            (src/c_api/c_api_profile.cc:264-560)
 //   Engine    the push/wait contract of include/mxnet/engine.h:115-314 (NewVariable / PushAsync / WaitForVar / WaitForAll) for C callbacks
 //   Storage   include/mxnet/storage.h Alloc / Free of the pooled host manager (src/storage/pooled_storage_manager.h:52-172)
-// Device tensors belong to PyTorch in this design (DESIGN.md §1), so an NDArray handle here owns HOST memory; device data crosses this ABI
-// through SyncCopy*.  Every function returns 0 on success and -1 on failure; GXRTGetLastError() describes the failure of the calling thread.
+// An NDArray handle owns host memory (GXNDArrayCreate) or float32 device memory from the native pool (GXNDArrayCreateEx, dev_type 2).  Work
+// on device arrays is ordered on one stream per device inside the kernel library: copies, executor passes and imperative operators are
+// enqueued in call order, and SyncCopyToCPU / WaitToRead / WaitToWrite / WaitAll synchronise that stream.  Every function returns 0 on
+// success and -1 on failure; GXRTGetLastError() describes the failure of the calling thread.
 #include <cstdint>
 #include <cstring>
 #include <fstream>
+#include <map>
+#include <set>
 #include <memory>
 #include <mutex>
 #include <string>
@@ -18,6 +22,7 @@
 
 #include "engine.h"
 #include "host_array.h"
+#include "kernel_lib.h"
 #include "params_io.h"
 #include "profiler.h"
 #include "storage.h"
@@ -52,6 +57,68 @@ gxrt::Engine* Eng() {
 GX_CAPI const char* GXRTGetLastError() { return rt_error.c_str(); }
 void GXRTSetLastError(const std::string& msg) { rt_error = msg; }       // for the other translation units of the C ABI (c_predict_api.cc)
 
+// ------------------------------------------------------------------------------------------------ device arrays
+namespace {
+std::mutex dev_mu;
+std::map<uintptr_t, size_t> dev_buffers;                                 // live device allocations: start -> bytes
+std::set<int> devices_used;
+}  // namespace
+namespace gxrt {
+namespace capi {
+size_t HostArray::Bytes() const { return device() ? static_cast<size_t>(gxrt::Prod(rec.shape)) * 4 : rec.data.size(); }
+HostArray* NewDeviceArray(const std::vector<int64_t>& shape, int dev) {
+  namespace K = gxrt::kern;
+  K::Stream s = K::DeviceStream(dev, "GXNDArrayCreateEx");
+  const K::Lib& L = K::Get();
+  auto a = std::make_unique<HostArray>();
+  a->rec.dtype = 0; a->rec.shape = shape; a->dev_id = dev;
+  const size_t bytes = static_cast<size_t>(gxrt::Prod(shape)) * 4;
+  K::Check(L.set_device(dev), "GXNDArrayCreateEx");
+  a->dptr = static_cast<float*>(L.pool_alloc(dev, bytes ? bytes : 4, s));
+  if (!a->dptr) throw std::runtime_error("GXNDArrayCreateEx: out of device memory on device " + std::to_string(dev) + " (" + std::to_string(bytes) + " bytes)");
+  a->owns_dptr = true;
+  { std::lock_guard<std::mutex> lk(dev_mu); dev_buffers[reinterpret_cast<uintptr_t>(a->dptr)] = bytes; devices_used.insert(dev); }
+  K::Check(L.memset(a->dptr, 0, bytes, s), "GXNDArrayCreateEx");
+  return a.release();
+}
+void ReleaseDevice(HostArray* a) {
+  if (!a->device() || !a->owns_dptr || !a->dptr) return;
+  { std::lock_guard<std::mutex> lk(dev_mu); dev_buffers.erase(reinterpret_cast<uintptr_t>(a->dptr)); }
+  const gxrt::kern::Lib& L = gxrt::kern::Get();
+  L.pool_free(a->dev_id, a->dptr, L.stream(a->dev_id));
+  a->dptr = nullptr;
+}
+gxrt::NDRec HostCopy(const HostArray* a) {
+  if (!a->device()) return a->rec;
+  namespace K = gxrt::kern;
+  gxrt::NDRec r;
+  r.dtype = a->rec.dtype; r.shape = a->rec.shape;
+  r.data.assign(a->Bytes(), '\0');
+  K::Stream s = K::Get().stream(a->dev_id);
+  K::Check(K::Get().memcpy(&r.data[0], a->dptr, r.data.size(), 2, s), "device -> host copy");
+  K::Check(K::Get().stream_sync(s), "device -> host copy");
+  return r;
+}
+void SyncDevice(int dev) {
+  namespace K = gxrt::kern;
+  K::Check(K::Get().stream_sync(K::Get().stream(dev)), "device synchronise");
+}
+void SyncAllDevices() {
+  std::set<int> devs;
+  { std::lock_guard<std::mutex> lk(dev_mu); devs = devices_used; }
+  for (int d : devs) SyncDevice(d);
+}
+bool IsDeviceBuffer(const void* p) {
+  const uintptr_t u = reinterpret_cast<uintptr_t>(p);
+  std::lock_guard<std::mutex> lk(dev_mu);
+  auto it = dev_buffers.upper_bound(u);
+  if (it == dev_buffers.begin()) return false;
+  --it;
+  return u < it->first + std::max<size_t>(it->second, 1);
+}
+}  // namespace capi
+}  // namespace gxrt
+
 // ------------------------------------------------------------------------------------------------ NDArray (host)
 // dtype: mshadow flags (0 f32, 1 f64, 2 f16, 3 u8, 4 i32, 5 i8, 6 i64)
 GX_CAPI int GXNDArrayCreate(const uint32_t* shape, uint32_t ndim, int dtype, void** out) {
@@ -61,6 +128,17 @@ GX_CAPI int GXNDArrayCreate(const uint32_t* shape, uint32_t ndim, int dtype, voi
     a->rec.shape.assign(shape, shape + ndim);
     a->rec.data.assign(static_cast<size_t>(gxrt::Prod(a->rec.shape)) * gxrt::FlagSize(dtype), '\0');
     *out = a.release();
+  });
+}
+// dev_type 1 (CPU): GXNDArrayCreate.  dev_type 2 (GPU): float32 device memory on dev_id from the native pool, zero-filled.  delay_alloc is
+// accepted for the reference's signature; memory is always allocated here.
+GX_CAPI int GXNDArrayCreateEx(const uint32_t* shape, uint32_t ndim, int dev_type, int dev_id, int delay_alloc, int dtype, void** out) {
+  (void)delay_alloc;
+  if (dev_type == 1) return GXNDArrayCreate(shape, ndim, dtype, out);
+  return Guard([&] {
+    if (dev_type != 2) throw std::runtime_error("GXNDArrayCreateEx: dev_type " + std::to_string(dev_type) + " is not supported (1 CPU, 2 GPU)");
+    if (dtype != 0) throw std::runtime_error("GXNDArrayCreateEx: device arrays are float32 (dtype flag 0), got dtype flag " + std::to_string(dtype));
+    *out = gxrt::capi::NewDeviceArray(std::vector<int64_t>(shape, shape + ndim), dev_id);
   });
 }
 GX_CAPI int GXNDArrayFree(void* h) { return Guard([&] { delete ND(h); }); }
@@ -73,12 +151,21 @@ GX_CAPI int GXNDArrayGetShape(void* h, uint32_t* out_ndim, const uint32_t** out_
   });
 }
 GX_CAPI int GXNDArrayGetDType(void* h, int* out) { return Guard([&] { *out = ND(h)->rec.dtype; }); }
-GX_CAPI int GXNDArrayGetData(void* h, void** out) { return Guard([&] { *out = &ND(h)->rec.data[0]; }); }
+// device arrays: the device pointer (for the caller's own CUDA code; work queued on the library stream may still be writing it — WaitToRead)
+GX_CAPI int GXNDArrayGetData(void* h, void** out) {
+  return Guard([&] { HostArray* a = ND(h); *out = a->device() ? static_cast<void*>(a->dptr) : static_cast<void*>(&a->rec.data[0]); });
+}
 GX_CAPI int GXNDArraySyncCopyFromCPU(void* h, const void* data, size_t size_elems) {
   return Guard([&] {
     HostArray* a = ND(h);
     const size_t bytes = size_elems * gxrt::FlagSize(a->rec.dtype);
-    if (bytes != a->rec.data.size()) throw std::runtime_error("SyncCopyFromCPU: size does not match the array");
+    if (bytes != a->Bytes()) throw std::runtime_error("SyncCopyFromCPU: size does not match the array");
+    if (a->device()) {
+      // pageable source: the copy has left `data` when cudaMemcpyAsync returns, so the caller may reuse its buffer at once
+      namespace K = gxrt::kern;
+      K::Check(K::Get().memcpy(a->dptr, data, bytes, 1, K::Get().stream(a->dev_id)), "SyncCopyFromCPU");
+      return;
+    }
     memcpy(&a->rec.data[0], data, bytes);
   });
 }
@@ -86,7 +173,14 @@ GX_CAPI int GXNDArraySyncCopyToCPU(void* h, void* data, size_t size_elems) {
   return Guard([&] {
     HostArray* a = ND(h);
     const size_t bytes = size_elems * gxrt::FlagSize(a->rec.dtype);
-    if (bytes != a->rec.data.size()) throw std::runtime_error("SyncCopyToCPU: size does not match the array");
+    if (bytes != a->Bytes()) throw std::runtime_error("SyncCopyToCPU: size does not match the array");
+    if (a->device()) {
+      namespace K = gxrt::kern;
+      K::Stream s = K::Get().stream(a->dev_id);
+      K::Check(K::Get().memcpy(data, a->dptr, bytes, 2, s), "SyncCopyToCPU");
+      K::Check(K::Get().stream_sync(s), "SyncCopyToCPU");
+      return;
+    }
     memcpy(data, a->rec.data.data(), bytes);
   });
 }
@@ -95,7 +189,7 @@ GX_CAPI int GXNDArraySave(const char* fname, uint32_t num, void** handles, const
   return Guard([&] {
     std::vector<gxrt::NDRec> recs;
     std::vector<std::string> names;
-    for (uint32_t i = 0; i < num; ++i) { recs.push_back(ND(handles[i])->rec); if (keys) names.emplace_back(keys[i]); }
+    for (uint32_t i = 0; i < num; ++i) { recs.push_back(gxrt::capi::HostCopy(ND(handles[i]))); if (keys) names.emplace_back(keys[i]); }
     const std::string blob = gxrt::WriteList(recs, names);
     std::ofstream f(fname, std::ios::binary);
     if (!f) throw std::runtime_error(std::string("cannot open ") + fname);

@@ -11,6 +11,7 @@
 #include <string>
 #include <vector>
 
+#include "host_array.h"
 #include "predict.h"
 #include "train_exec.h"
 
@@ -233,14 +234,20 @@ GX_CAPI int GXPredGetNumOutputs(void* handle, uint32_t* out) {
   return Guard([&] { Handle* h = H(handle); *out = static_cast<uint32_t>(h->pred ? h->pred->NumOutputs() : h->gen->NumOutputs()); });
 }
 GX_CAPI int GXPredSetInput(void* handle, const char* key, const float* data, uint32_t size) {
-  return Guard([&] { Handle* h = H(handle); if (h->pred) h->pred->SetInput(key, data, size); else h->gen->SetInput(key, data, size); });
+  return Guard([&] {
+    if (gxrt::capi::IsDeviceBuffer(data)) throw std::runtime_error("GXPredSetInput: device array (the predictor reads host memory; serve device data through GXExecutorForward)");
+    Handle* h = H(handle); if (h->pred) h->pred->SetInput(key, data, size); else h->gen->SetInput(key, data, size);
+  });
 }
 GX_CAPI int GXPredForward(void* handle) { return Guard([&] { Handle* h = H(handle); if (h->pred) h->pred->Forward(); else h->gen->Forward(); }); }
 GX_CAPI int GXPredPartialForward(void* handle, int step, int* step_left) {
   return Guard([&] { Handle* h = H(handle); if (h->pred) h->pred->PartialForward(step, step_left); else h->gen->PartialForward(step, step_left); });
 }
 GX_CAPI int GXPredGetOutput(void* handle, uint32_t index, float* data, uint32_t size) {
-  return Guard([&] { Handle* h = H(handle); if (h->pred) h->pred->GetOutput(index, data, size); else h->gen->GetOutput(index, data, size); });
+  return Guard([&] {
+    if (gxrt::capi::IsDeviceBuffer(data)) throw std::runtime_error("GXPredGetOutput: device array (the predictor writes host memory)");
+    Handle* h = H(handle); if (h->pred) h->pred->GetOutput(index, data, size); else h->gen->GetOutput(index, data, size);
+  });
 }
 // 1: the planned predictor (predict.h) runs this graph, 2: the general executor (train_exec.h) does
 GX_CAPI int GXPredGetEngine(void* handle, int* out) { return Guard([&] { *out = H(handle)->pred ? 1 : 2; }); }

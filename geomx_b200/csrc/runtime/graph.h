@@ -130,6 +130,9 @@ inline std::vector<std::string> InTake(const AttrView&) { return {"a", "indices"
 inline std::vector<std::string> InPick(const AttrView&) { return {"data", "index"}; }
 inline std::vector<std::string> InWhere(const AttrView&) { return {"condition", "x", "y"}; }
 inline std::vector<std::string> InIdx(const AttrView&) { return {"indices"}; }
+inline std::vector<std::string> InSGD(const AttrView&) { return {"weight", "grad"}; }
+inline std::vector<std::string> InSGDMom(const AttrView&) { return {"weight", "grad", "mom"}; }
+inline std::vector<std::string> InAdam(const AttrView&) { return {"weight", "grad", "mean", "var"}; }
 inline std::vector<std::string> InVar(const AttrView& a) {
   std::vector<std::string> v;
   const int64_t n = a.Int("num_args", 0);
@@ -185,6 +188,17 @@ inline const std::vector<OpDef>& OpTable() {
     v.push_back({"LinearRegressionOutput", InDataLabel, 0, "", "identity forward, (x - y) backward (src/operator/regression_output.cc)", {{"grad_scale", "float, optional, default=1", "gradient scale"}}});
     v.push_back({"LogisticRegressionOutput", InDataLabel, 0, "", "sigmoid forward, (p - y) backward", {{"grad_scale", "float, optional, default=1", "gradient scale"}}});
     v.push_back({"MAERegressionOutput", InDataLabel, 0, "", "identity forward, sign(x - y) backward", {{"grad_scale", "float, optional, default=1", "gradient scale"}}});
+    // optimizer steps for imperative use: the output is the updated weight, optimizer states are trailing auxiliary inputs updated in place
+    const std::vector<ParamDoc> opt_common = {{"lr", "float, required", "learning rate"}, {"wd", "float, optional, default=0", "weight decay"},
+                                              {"rescale_grad", "float, optional, default=1", "gradient scale"},
+                                              {"clip_gradient", "float, optional, default=-1", "clip the rescaled gradient to +-value (< 0: off)"}};
+    auto with = [&](std::vector<ParamDoc> extra) { std::vector<ParamDoc> p = opt_common; p.insert(p.end(), extra.begin(), extra.end()); return p; };
+    v.push_back({"sgd_update", InSGD, 0, "", "w - lr * (clip(rescale_grad * g) + wd * w) (src/operator/optimizer_op.cc)", opt_common});
+    v.push_back({"sgd_mom_update", InSGDMom, 1, "", "mom = momentum * mom - lr * (clip(rescale_grad * g) + wd * w); w + mom (src/operator/optimizer_op.cc)",
+                 with({{"momentum", "float, optional, default=0", "momentum"}})});
+    v.push_back({"adam_update", InAdam, 2, "", "Adam step without bias correction on (weight, grad, mean, var) (src/operator/optimizer_op.cc)",
+                 with({{"beta1", "float, optional, default=0.9", "first-moment decay"}, {"beta2", "float, optional, default=0.999", "second-moment decay"},
+                       {"epsilon", "float, optional, default=1e-8", "denominator floor"}})});
     v.push_back({"MakeLoss", InData, 0, "", "marks a head as a loss: backward feeds grad_scale (src/operator/make_loss.cc)", {{"grad_scale", "float, optional, default=1", "gradient scale"}}});
     v.push_back({"softmax", InData, 0, "", "softmax along an axis (src/operator/nn/softmax.cc)", {{"axis", "int, optional, default=-1", "axis"}}});
     v.push_back({"log_softmax", InData, 0, "", "log-softmax along an axis", {{"axis", "int, optional, default=-1", "axis"}}});
@@ -718,7 +732,7 @@ inline bool InferNode(const Node& n, const std::vector<const Shape*>& in, const 
       o[ax] += s[ax];
     }
     *out = o;
-  } else if (op == "add_n") {
+  } else if (op == "add_n" || op == "sgd_update" || op == "sgd_mom_update" || op == "adam_update") {
     for (size_t i = 1; i < in.size(); ++i) need(i, x);
     *out = x;
   } else if (op == "Embedding") {

@@ -7,7 +7,8 @@
 // (src/operator/nn/*.cc, src/operator/softmax_output-inl.h, regression_output-inl.h).  The reference builds a separate backward graph with
 // nnvm::pass::Gradient and plans memory for both; here the forward activations are kept per node and the backward pass is a reverse sweep
 // that calls one gradient routine per operator — on the host the simplicity is worth more than the reuse (the device path's equivalents are
-// the fused sm_100a kernels and the CUDA-graph executor of models/cnn.py, DESIGN.md §1).
+// the fused sm_100a kernels and the CUDA-graph executor of models/cnn.py, DESIGN.md §1).  Its device twin for graphs bound to device arrays
+// of the C API is device_exec.h::DeviceExecutor: same slot layout and gradient-flow rules, sm_100a kernels per node.
 #pragma once
 #include <atomic>
 #include <cstring>
@@ -454,6 +455,26 @@ class Executor {
     } else if (op == "add_n") {
       memcpy(y, x, ny * sizeof(float));
       for (size_t k = 1; k < s.in.size(); ++k) { const float* v = Val(s.in[k]); for (int64_t i = 0; i < ny; ++i) y[i] += v[i]; }
+    } else if (op == "sgd_update" || op == "sgd_mom_update" || op == "adam_update") {
+      // ndarray/op_lib.py: g = clip(rescale * grad) + wd * w; the states (trailing auxiliary inputs) are updated in place
+      const float lr = static_cast<float>(a.Float("lr", 0)), wd = static_cast<float>(a.Float("wd", 0)), rescale = static_cast<float>(a.Float("rescale_grad", 1)),
+                  clip = static_cast<float>(a.Float("clip_gradient", -1));
+      const float* g = Val(s.in[1]);
+      auto prep = [&](int64_t i) { float v = g[i] * rescale; if (clip >= 0.f) v = std::min(std::max(v, -clip), clip); return v + wd * x[i]; };
+      if (op == "sgd_update") for (int64_t i = 0; i < ny; ++i) y[i] = x[i] - lr * prep(i);
+      else if (op == "sgd_mom_update") {
+        const float mom = static_cast<float>(a.Float("momentum", 0));
+        float* m = AuxPtr(s.in[2]);
+        for (int64_t i = 0; i < ny; ++i) { m[i] = m[i] * mom - lr * prep(i); y[i] = x[i] + m[i]; }
+      } else {
+        const float b1 = static_cast<float>(a.Float("beta1", 0.9)), b2 = static_cast<float>(a.Float("beta2", 0.999)), eps = static_cast<float>(a.Float("epsilon", 1e-8));
+        float* m = AuxPtr(s.in[2]); float* v = AuxPtr(s.in[3]);
+        for (int64_t i = 0; i < ny; ++i) {
+          const float gg = prep(i);
+          m[i] = m[i] * b1 + gg * (1.f - b1); v[i] = v[i] * b2 + gg * gg * (1.f - b2);
+          y[i] = x[i] - lr * m[i] / (std::sqrt(v[i]) + eps);
+        }
+      }
     } else if (op == "Embedding") {
       const float* w = Val(s.in[1]);
       const int64_t V = slots_[s.in[1]].shape[0], D = slots_[s.in[1]].shape[1];
@@ -989,7 +1010,7 @@ class Executor {
     } else if (op == "where") {
       float* dt = GradOf(s.in[1]); float* df = GradOf(s.in[2]);
       for (int64_t i = 0; i < ny; ++i) { if (x[i] != 0.f) { if (dt) dt[i] += dy[i]; } else if (df) df[i] += dy[i]; }
-    } else if (op == "one_hot" || op == "argmax" || op == "argmin") {
+    } else if (op == "one_hot" || op == "argmax" || op == "argmin" || op == "sgd_update" || op == "sgd_mom_update" || op == "adam_update") {
     } else if (op == "max" || op == "min" || op == "prod" || op == "norm") {
       if (!dx) return;
       const auto red = ReducedAxes(s, xs);

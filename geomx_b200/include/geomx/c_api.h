@@ -6,9 +6,14 @@
  * failure of the calling thread is GXRTGetLastError() (KVStore group: GXGetLastError()).  Returned string / array pointers live in
  * thread-local storage of the library and stay valid until the next call of the same function group on the same thread.
  *
- * What executes where: NDArray handles of this ABI own HOST memory and the Symbol / Executor / autograd groups compute in float32 on the
- * host (csrc/runtime/train_exec.h) — the path to train or serve without PyTorch in the process.  Device execution (sm_100a kernels, CUDA
- * graphs, the NVLink fabric) is driven from the Python package; GXKVStore* is the TCP parameter-server plane both share.
+ * What executes where: an NDArray handle owns HOST memory (GXNDArrayCreate, GXNDArrayCreateEx with dev_type 1) or float32 DEVICE memory
+ * (GXNDArrayCreateEx with dev_type 2, from the native pool).  Executors bound to host arrays compute in float32 on the host
+ * (csrc/runtime/train_exec.h); executors bound to device arrays (GXExecutorSimpleBindEx / GXExecutorBind with dev_type 2) and imperative
+ * calls on device arrays run sm_100a kernels of libgeomx_kernels.so (csrc/runtime/device_exec.h), which this library loads at the first
+ * device request from its own directory — it has no link-time dependency on CUDA.  Device work is ordered on one stream per device in call
+ * order; SyncCopyToCPU and the Wait* functions synchronise it.  Functions that read host bytes (Slice / At / Reshape / Detach, autograd,
+ * GXKVStore*, GXPred*) refuse device arrays.  CUDA graphs, the NVLink fabric and mixed precision are driven from the Python package;
+ * GXKVStore* is the TCP parameter-server plane both share.
  *
  * dtype flags: 0 float32, 1 float64, 2 float16, 3 uint8, 4 int32, 5 int8, 6 int64.  grad_req: 0 null, 1 write, 3 add.
  */
@@ -39,8 +44,11 @@ const char* GXGetLastError(void);                       /* KVStore group */
 int GXGetVersion(int* out);
 int GXRandomSeed(int seed);
 
-/* ---- NDArray (host) ------------------------------------------------------------------------------------------------------------------ */
-int GXNDArrayCreate(const uint32_t* shape, uint32_t ndim, int dtype, NDArrayHandle* out);
+/* ---- NDArray ------------------------------------------------------------------------------------------------------------------------- */
+int GXNDArrayCreate(const uint32_t* shape, uint32_t ndim, int dtype, NDArrayHandle* out);                                       /* host */
+/* dev_type 1 CPU (= GXNDArrayCreate), 2 GPU: float32 device memory on dev_id (zero-filled); GetData then returns the device pointer,
+ * GetContext (2, dev_id), SyncCopy* copy host <-> device, Save / SaveRawBytes copy to the host first */
+int GXNDArrayCreateEx(const uint32_t* shape, uint32_t ndim, int dev_type, int dev_id, int delay_alloc, int dtype, NDArrayHandle* out);
 int GXNDArrayFree(NDArrayHandle h);
 int GXNDArrayGetShape(NDArrayHandle h, uint32_t* out_ndim, const uint32_t** out_shape);
 int GXNDArrayGetDType(NDArrayHandle h, int* out);
@@ -103,7 +111,7 @@ int GXSymbolInferShapePartial(SymbolHandle sym, uint32_t num_args, const char** 
 int GXSymbolInferType(SymbolHandle sym, uint32_t num_args, const char** keys, const int* arg_type_data, uint32_t* in_type_size, const int** in_type_data,
                       uint32_t* out_type_size, const int** out_type_data, uint32_t* aux_type_size, const int** aux_type_data, int* complete);
 
-/* ---- Executor (host, float32) -------------------------------------------------------------------------------------------------------- */
+/* ---- Executor (float32; host arrays: host executor, device arrays: device executor) --------------------------------------------------- */
 int GXExecutorBind(SymbolHandle sym, int dev_type, int dev_id, uint32_t len, NDArrayHandle* in_args, NDArrayHandle* arg_grad_store, const uint32_t* grad_req_type,
                    uint32_t aux_states_len, NDArrayHandle* aux_states, ExecutorHandle* out);
 /* allocates arguments / gradients / auxiliary states from the given input shapes; grad_req "null" | "write" | "add" for every argument
@@ -111,6 +119,11 @@ int GXExecutorBind(SymbolHandle sym, int dev_type, int dev_id, uint32_t len, NDA
 int GXExecutorSimpleBind(SymbolHandle sym, uint32_t num_shapes, const char** keys, const uint32_t* ind_ptr, const uint32_t* shape_data, const char* grad_req,
                          uint32_t num_no_grad, const char** no_grad_keys, ExecutorHandle* out, uint32_t* num_args, NDArrayHandle** in_args, NDArrayHandle** arg_grads,
                          uint32_t* num_aux, NDArrayHandle** aux_states);
+/* the same with a device: dev_type 1 = GXExecutorSimpleBind; dev_type 2 allocates device arrays on dev_id and binds the device executor,
+ * whose Outputs are device arrays.  Operators outside the device set are refused here with the node's name. */
+int GXExecutorSimpleBindEx(SymbolHandle sym, int dev_type, int dev_id, uint32_t num_shapes, const char** keys, const uint32_t* ind_ptr, const uint32_t* shape_data,
+                           const char* grad_req, uint32_t num_no_grad, const char** no_grad_keys, ExecutorHandle* out, uint32_t* num_args, NDArrayHandle** in_args,
+                           NDArrayHandle** arg_grads, uint32_t* num_aux, NDArrayHandle** aux_states);
 int GXExecutorForward(ExecutorHandle h, int is_train);
 int GXExecutorBackward(ExecutorHandle h, uint32_t len, NDArrayHandle* head_grads);       /* len 0 for loss heads */
 int GXExecutorBackwardEx(ExecutorHandle h, uint32_t len, NDArrayHandle* head_grads, int is_train);
@@ -118,7 +131,9 @@ int GXExecutorOutputs(ExecutorHandle h, uint32_t* out_size, NDArrayHandle** out)
 int GXExecutorPrint(ExecutorHandle h, const char** out_str);
 int GXExecutorFree(ExecutorHandle h);
 
-/* ---- imperative invoke + autograd ---------------------------------------------------------------------------------------------------- */
+/* ---- imperative invoke + autograd ----------------------------------------------------------------------------------------------------
+ * Device inputs run the operator on their device (outputs: device arrays on the same device, which may alias an input); sgd_update,
+ * sgd_mom_update and adam_update take the optimizer states as trailing inputs and update them in place.  Autograd records host arrays only. */
 int GXImperativeInvoke(AtomicSymbolCreator creator, int num_inputs, NDArrayHandle* inputs, int* num_outputs, NDArrayHandle** outputs, int num_params,
                        const char** param_keys, const char** param_vals);
 int GXImperativeInvokeByName(const char* op, int num_inputs, NDArrayHandle* inputs, int* num_outputs, NDArrayHandle** outputs, int num_params,
