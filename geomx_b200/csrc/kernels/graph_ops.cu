@@ -5,7 +5,8 @@
 // executor zeroes gradients once per Backward and fan-out accumulates, as in the host executor (train_exec.h).
 //
 // The gx_rt_* functions give the C API (compiled with g++, without CUDA headers, loading this library with dlopen) the few runtime calls it
-// needs: device count, current device, one stream per device, copies, memset and stream synchronisation.
+// needs: device count, current device, one stream per device, streams of its own (one per native predictor), copies, memset, stream
+// synchronisation and the capture / replay of a stream's work as a CUDA graph.
 #include <cuda_runtime.h>
 
 #include <mutex>
@@ -129,7 +130,7 @@ __global__ void pool_bwd_kernel(const float* __restrict__ dy, const int* __restr
   }
 }
 
-// ------------------------------------------------------------------------------------------------ broadcast binary (add / sub / mul)
+// ------------------------------------------------------------------------------------------------ broadcast binary (add / sub / mul / div / max / min)
 constexpr int kMaxDims = 8;
 struct Bcast { int ndim; long long dims[kMaxDims], ls[kMaxDims], rs[kMaxDims]; };   // output extents; operand strides (0 on broadcast axes)
 
@@ -138,7 +139,17 @@ __device__ __forceinline__ void bcast_offsets(const Bcast& b, long long f, long 
   for (int d = b.ndim - 1; d >= 0; --d) { const long long c = f % b.dims[d]; f /= b.dims[d]; l += c * b.ls[d]; r += c * b.rs[d]; }
   *li = l; *ri = r;
 }
-__device__ __forceinline__ float bin_f(int k, float l, float r) { return k == 0 ? l + r : k == 1 ? l - r : l * r; }
+// 3 div, 4 maximum, 5 minimum (forward only; the operands' order in 4 / 5 is std::max / std::min's)
+__device__ __forceinline__ float bin_f(int k, float l, float r) {
+  switch (k) {
+    case 0: return l + r;
+    case 1: return l - r;
+    case 2: return l * r;
+    case 3: return l / r;
+    case 4: return l < r ? r : l;
+    default: return r < l ? r : l;
+  }
+}
 
 __global__ void binary_fwd_kernel(int kind, const float* __restrict__ l, const float* __restrict__ r, float* __restrict__ y, long long n, Bcast b) {
   pdl_wait();
@@ -317,9 +328,9 @@ GX_API void* gx_rt_stream(int dev) {
   }
   return g_streams[dev];
 }
-// kind: 1 host -> device, 2 device -> host, 3 device -> device; ordered on `stream`
+// kind: 1 host -> device, 2 device -> host, 3 device -> device, 4 inferred from the pointers (cudaMemcpyDefault); ordered on `stream`
 GX_API int gx_rt_memcpy(void* dst, const void* src, unsigned long long bytes, int kind, void* stream) {
-  const cudaMemcpyKind k = kind == 1 ? cudaMemcpyHostToDevice : kind == 2 ? cudaMemcpyDeviceToHost : cudaMemcpyDeviceToDevice;
+  const cudaMemcpyKind k = kind == 1 ? cudaMemcpyHostToDevice : kind == 2 ? cudaMemcpyDeviceToHost : kind == 4 ? cudaMemcpyDefault : cudaMemcpyDeviceToDevice;
   if (bytes == 0) return 0;
   return (int)cudaMemcpyAsync(dst, src, bytes, k, static_cast<cudaStream_t>(stream));
 }
@@ -329,6 +340,38 @@ GX_API int gx_rt_memset(void* dst, int value, unsigned long long bytes, void* st
 }
 GX_API int gx_rt_stream_sync(void* stream) { return (int)cudaStreamSynchronize(static_cast<cudaStream_t>(stream)); }
 GX_API const char* gx_rt_error_string(int code) { return cudaGetErrorString(static_cast<cudaError_t>(code)); }
+// a non-blocking stream on `dev` owned by the caller (the current device is left as it was)
+GX_API int gx_rt_stream_create(int dev, void** out) {
+  *out = nullptr;
+  int cur = 0;
+  cudaGetDevice(&cur);
+  cudaError_t e = cudaSetDevice(dev);
+  cudaStream_t s = nullptr;
+  if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&s, cudaStreamNonBlocking);
+  cudaSetDevice(cur);
+  if (e != cudaSuccess) { cudaGetLastError(); return (int)e; }
+  *out = s;
+  return 0;
+}
+GX_API int gx_rt_stream_destroy(void* stream) { return stream ? (int)cudaStreamDestroy(static_cast<cudaStream_t>(stream)) : 0; }
+// CUDA graphs of one stream's work.  Capture is thread-local: allocations and other calls made meanwhile by other threads (another
+// predictor's create, the pool's cudaMalloc) neither join nor invalidate it.
+GX_API int gx_rt_graph_begin(void* stream) { return (int)cudaStreamBeginCapture(static_cast<cudaStream_t>(stream), cudaStreamCaptureModeThreadLocal); }
+// ends the capture and instantiates it; on failure *out is null and the capture is over
+GX_API int gx_rt_graph_end(void* stream, void** out) {
+  *out = nullptr;
+  cudaGraph_t g = nullptr;
+  cudaError_t e = cudaStreamEndCapture(static_cast<cudaStream_t>(stream), &g);
+  if (e != cudaSuccess) { cudaGetLastError(); if (g) cudaGraphDestroy(g); return (int)e; }
+  cudaGraphExec_t x = nullptr;
+  e = cudaGraphInstantiateWithFlags(&x, g, 0);
+  cudaGraphDestroy(g);
+  if (e != cudaSuccess) { cudaGetLastError(); return (int)e; }
+  *out = x;
+  return 0;
+}
+GX_API int gx_rt_graph_launch(void* exec, void* stream) { return (int)cudaGraphLaunch(static_cast<cudaGraphExec_t>(exec), static_cast<cudaStream_t>(stream)); }
+GX_API int gx_rt_graph_destroy(void* exec) { return exec ? (int)cudaGraphExecDestroy(static_cast<cudaGraphExec_t>(exec)) : 0; }
 
 // ================================================================================================ graph operator kernels
 GX_API int gx_axpy(float* y, const float* x, float a, long long n, cudaStream_t s) {
@@ -367,10 +410,11 @@ GX_API int gx_pool_bwd(int type, const float* dy, const int* idx, float* dx, lon
   const PoolGeom g{H, W, OH, OW, kh, kw, sh, sw, ph, pw, type, count_pad};
   return launch_pdl(pool_bwd_kernel, dim3(blocks_for(NC * OH * OW)), dim3(kThreads), 0, s, dy, idx, dx, NC, g);
 }
-// kind 0 add, 1 sub, 2 mul.  out_dims: the output extents (ndim <= 8); ls / rs: element strides of each operand, 0 on broadcast axes
+// kind 0 add, 1 sub, 2 mul, 3 div, 4 maximum, 5 minimum (gx_binary_bwd: 0-2).  out_dims: the output extents (ndim <= 8); ls / rs: element
+// strides of each operand, 0 on broadcast axes
 GX_API int gx_binary_fwd(int kind, const float* l, const float* r, float* y, int ndim, const long long* out_dims, const long long* ls, const long long* rs,
                          cudaStream_t s) {
-  if (kind < 0 || kind > 2 || ndim < 1 || ndim > kMaxDims) return -1;
+  if (kind < 0 || kind > 5 || ndim < 1 || ndim > kMaxDims) return -1;
   Bcast b; b.ndim = ndim;
   long long n = 1;
   for (int d = 0; d < ndim; ++d) { b.dims[d] = out_dims[d]; b.ls[d] = ls[d]; b.rs[d] = rs[d]; n *= out_dims[d]; }

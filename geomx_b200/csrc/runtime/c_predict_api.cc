@@ -3,7 +3,9 @@
 // Parity (GX prefix, same argument lists): include/mxnet/c_predict_api.h
 //   MXPredCreate :78, MXPredCreatePartialOut :111, MXPredCreateMultiThread :144, MXPredReshape :170, MXPredGetOutputShape :185,
 //   MXPredSetInput :198, MXPredForward :207, MXPredPartialForward :224, MXPredGetOutput :233, MXPredFree :242, MXNDList{Create,Get,Free} :252-277.
-// dev_type 1 (cpu) runs here; dev_type 2 is refused with a message — device inference goes through the Python Executor on PyTorch tensors.
+// dev_type 1 (cpu) runs on the host: the planned predictor (predict.h), or the general executor for graphs outside its operator set.
+// dev_type 2 (gpu) runs the planned predictor on device dev_id with sm_100a kernels (predict_device.h); there is no host fallback, and a
+// graph the device runner cannot serve is refused at create.
 // Errors: -1 + GXRTGetLastError() (shared with c_api_runtime.cc, thread-local).
 #include <cstdint>
 #include <map>
@@ -13,6 +15,7 @@
 
 #include "host_array.h"
 #include "predict.h"
+#include "predict_device.h"
 #include "train_exec.h"
 
 #define GX_CAPI extern "C" __attribute__((visibility("default")))
@@ -21,6 +24,7 @@ extern "C" const char* GXRTGetLastError();
 void GXRTSetLastError(const std::string& msg);          // c_api_runtime.cc
 
 namespace {
+using gxrt::predict::DevicePredictor;
 using gxrt::predict::NDList;
 using gxrt::predict::Predictor;
 using gxrt::predict::Shape;
@@ -143,10 +147,25 @@ class GraphPredictor {
 
 struct Handle {
   std::unique_ptr<Predictor> pred;       // the planned predictor (predict.h) ...
-  std::unique_ptr<GraphPredictor> gen;   // ... or the general executor, when the graph needs operators the planned one does not have
+  std::unique_ptr<GraphPredictor> gen;   // ... or the general executor, when the graph needs operators the planned one does not have ...
+  std::unique_ptr<DevicePredictor> dev;  // ... or the planned predictor on a GPU (dev_type 2)
   std::vector<uint32_t> shape_out;       // GetOutputShape hands out a pointer that stays valid until the next call on this handle
+  const gxrt::predict::GraphPlan& plan() const { if (dev) return *dev; if (pred) return *pred; throw std::logic_error("no planned predictor"); }
 };
 Handle* H(void* h) { if (!h) throw std::runtime_error("null predictor handle"); return static_cast<Handle*>(h); }
+// a device handle makes its device current before anything else
+Handle* HD(void* h, const char* fn) { Handle* x = H(h); if (x->dev) x->dev->SetDevice(fn); return x; }
+// a create: every error on a GPU also says where graphs the native device runner cannot serve can go instead
+template <typename F>
+int CreateGuard(int dev_type, F&& f) {
+  return Guard([&] {
+    try { f(); }
+    catch (const std::exception& e) {
+      if (dev_type != 2) throw;
+      throw std::runtime_error(e.what() + std::string("; geomx_b200.predictor.Predictor(dev_type='gpu') serves graphs on the Python Executor"));
+    }
+  });
+}
 
 std::vector<Shape> Shapes(uint32_t n, const uint32_t* indptr, const uint32_t* data) {
   std::vector<Shape> out(n);
@@ -156,15 +175,19 @@ std::vector<Shape> Shapes(uint32_t n, const uint32_t* indptr, const uint32_t* da
   }
   return out;
 }
-void Make(Handle* h, const char* json, const void* params, int param_size, int dev_type, uint32_t n_in, const char** keys,
+void Make(Handle* h, const char* json, const void* params, int param_size, int dev_type, int dev_id, uint32_t n_in, const char** keys,
           const uint32_t* indptr, const uint32_t* shape_data, uint32_t n_out, const char** out_keys) {
-  if (dev_type != 1) throw std::runtime_error("the native predictor runs on the host (dev_type 1); use the Python Executor for device inference");
+  if (dev_type != 1 && dev_type != 2) throw std::runtime_error("dev_type " + std::to_string(dev_type) + " is not supported (1 CPU, 2 GPU)");
   if (json == nullptr) throw std::runtime_error("null symbol JSON");
   if (param_size < 0) throw std::runtime_error("negative param_size");
   std::vector<std::string> ik, ok;
   for (uint32_t i = 0; i < n_in; ++i) ik.emplace_back(keys[i]);
   for (uint32_t i = 0; i < n_out; ++i) ok.emplace_back(out_keys[i]);
   const auto shapes = Shapes(n_in, indptr, shape_data);
+  if (dev_type == 2) {
+    h->dev = std::make_unique<DevicePredictor>(std::string(json), static_cast<const char*>(params), static_cast<size_t>(param_size), ik, shapes, ok, dev_id);
+    return;
+  }
   try {
     h->pred = std::make_unique<Predictor>(std::string(json), static_cast<const char*>(params), static_cast<size_t>(param_size), ik, shapes, ok);
   } catch (const std::runtime_error& e) {
@@ -178,34 +201,38 @@ void Make(Handle* h, const char* json, const void* params, int param_size, int d
 }
 }  // namespace
 
-GX_CAPI int GXPredCreate(const char* symbol_json, const void* param_bytes, int param_size, int dev_type, int /*dev_id*/, uint32_t num_input_nodes,
+GX_CAPI int GXPredCreate(const char* symbol_json, const void* param_bytes, int param_size, int dev_type, int dev_id, uint32_t num_input_nodes,
                          const char** input_keys, const uint32_t* input_shape_indptr, const uint32_t* input_shape_data, void** out) {
-  return Guard([&] {
+  return CreateGuard(dev_type, [&] {
     auto h = std::make_unique<Handle>();
-    Make(h.get(), symbol_json, param_bytes, param_size, dev_type, num_input_nodes, input_keys, input_shape_indptr, input_shape_data, 0, nullptr);
+    Make(h.get(), symbol_json, param_bytes, param_size, dev_type, dev_id, num_input_nodes, input_keys, input_shape_indptr, input_shape_data, 0, nullptr);
     *out = h.release();
   });
 }
-GX_CAPI int GXPredCreatePartialOut(const char* symbol_json, const void* param_bytes, int param_size, int dev_type, int /*dev_id*/, uint32_t num_input_nodes,
+GX_CAPI int GXPredCreatePartialOut(const char* symbol_json, const void* param_bytes, int param_size, int dev_type, int dev_id, uint32_t num_input_nodes,
                                    const char** input_keys, const uint32_t* input_shape_indptr, const uint32_t* input_shape_data,
                                    uint32_t num_output_nodes, const char** output_keys, void** out) {
-  return Guard([&] {
+  return CreateGuard(dev_type, [&] {
     auto h = std::make_unique<Handle>();
-    Make(h.get(), symbol_json, param_bytes, param_size, dev_type, num_input_nodes, input_keys, input_shape_indptr, input_shape_data, num_output_nodes, output_keys);
+    Make(h.get(), symbol_json, param_bytes, param_size, dev_type, dev_id, num_input_nodes, input_keys, input_shape_indptr, input_shape_data, num_output_nodes,
+         output_keys);
     *out = h.release();
   });
 }
-// num_threads predictors over ONE copy of the graph and the parameters, each with its own inputs and activation arena
-GX_CAPI int GXPredCreateMultiThread(const char* symbol_json, const void* param_bytes, int param_size, int dev_type, int /*dev_id*/, uint32_t num_input_nodes,
+// num_threads predictors over ONE copy of the graph and the parameters, each with its own inputs and activation arena (and, on a GPU, its
+// own stream: the handles may serve from different threads at once)
+GX_CAPI int GXPredCreateMultiThread(const char* symbol_json, const void* param_bytes, int param_size, int dev_type, int dev_id, uint32_t num_input_nodes,
                                     const char** input_keys, const uint32_t* input_shape_indptr, const uint32_t* input_shape_data, int num_threads, void** out) {
-  return Guard([&] {
+  return CreateGuard(dev_type, [&] {
     if (num_threads < 1) throw std::runtime_error("num_threads must be positive");
     std::vector<std::unique_ptr<Handle>> hs;
     hs.push_back(std::make_unique<Handle>());
-    Make(hs[0].get(), symbol_json, param_bytes, param_size, dev_type, num_input_nodes, input_keys, input_shape_indptr, input_shape_data, 0, nullptr);
+    Make(hs[0].get(), symbol_json, param_bytes, param_size, dev_type, dev_id, num_input_nodes, input_keys, input_shape_indptr, input_shape_data, 0, nullptr);
     for (int i = 1; i < num_threads; ++i) {
       hs.push_back(std::make_unique<Handle>());
-      if (hs[0]->pred) hs[i]->pred = hs[0]->pred->Clone(nullptr); else hs[i]->gen = hs[0]->gen->Clone(nullptr);
+      if (hs[0]->dev) hs[i]->dev = hs[0]->dev->Clone(nullptr);
+      else if (hs[0]->pred) hs[i]->pred = hs[0]->pred->Clone(nullptr);
+      else hs[i]->gen = hs[0]->gen->Clone(nullptr);
     }
     for (int i = 0; i < num_threads; ++i) out[i] = hs[i].release();
   });
@@ -217,49 +244,66 @@ GX_CAPI int GXPredReshape(uint32_t num_input_nodes, const char** input_keys, con
     const auto list = Shapes(num_input_nodes, input_shape_indptr, input_shape_data);
     for (uint32_t i = 0; i < num_input_nodes; ++i) shapes[input_keys[i]] = list[i];
     auto h = std::make_unique<Handle>();
-    if (H(handle)->pred) h->pred = H(handle)->pred->Clone(&shapes); else h->gen = H(handle)->gen->Clone(&shapes);
+    Handle* src = HD(handle, "GXPredReshape");
+    if (src->dev) h->dev = src->dev->Clone(&shapes);
+    else if (src->pred) h->pred = src->pred->Clone(&shapes);
+    else h->gen = src->gen->Clone(&shapes);
     *out = h.release();
   });
 }
 GX_CAPI int GXPredGetOutputShape(void* handle, uint32_t index, uint32_t** shape_data, uint32_t* shape_ndim) {
   return Guard([&] {
-    Handle* h = H(handle);
-    const Shape& s = h->pred ? h->pred->OutputShape(index) : h->gen->OutputShape(index);
+    Handle* h = HD(handle, "GXPredGetOutputShape");
+    const Shape& s = h->gen ? h->gen->OutputShape(index) : h->plan().OutputShape(index);
     h->shape_out.assign(s.begin(), s.end());
     *shape_data = h->shape_out.data();
     *shape_ndim = static_cast<uint32_t>(h->shape_out.size());
   });
 }
 GX_CAPI int GXPredGetNumOutputs(void* handle, uint32_t* out) {
-  return Guard([&] { Handle* h = H(handle); *out = static_cast<uint32_t>(h->pred ? h->pred->NumOutputs() : h->gen->NumOutputs()); });
+  return Guard([&] { Handle* h = HD(handle, "GXPredGetNumOutputs"); *out = static_cast<uint32_t>(h->gen ? h->gen->NumOutputs() : h->plan().NumOutputs()); });
 }
+// host handles read host memory only; device handles (dev_type 2) read host or device memory
 GX_CAPI int GXPredSetInput(void* handle, const char* key, const float* data, uint32_t size) {
   return Guard([&] {
-    if (gxrt::capi::IsDeviceBuffer(data)) throw std::runtime_error("GXPredSetInput: device array (the predictor reads host memory; serve device data through GXExecutorForward)");
-    Handle* h = H(handle); if (h->pred) h->pred->SetInput(key, data, size); else h->gen->SetInput(key, data, size);
+    if ((!handle || !H(handle)->dev) && gxrt::capi::IsDeviceBuffer(data))
+      throw std::runtime_error("GXPredSetInput: device array (the predictor reads host memory; serve device data through GXExecutorForward)");
+    Handle* h = HD(handle, "GXPredSetInput");
+    if (h->dev) h->dev->SetInput(key, data, size); else if (h->pred) h->pred->SetInput(key, data, size); else h->gen->SetInput(key, data, size);
   });
 }
-GX_CAPI int GXPredForward(void* handle) { return Guard([&] { Handle* h = H(handle); if (h->pred) h->pred->Forward(); else h->gen->Forward(); }); }
-GX_CAPI int GXPredPartialForward(void* handle, int step, int* step_left) {
-  return Guard([&] { Handle* h = H(handle); if (h->pred) h->pred->PartialForward(step, step_left); else h->gen->PartialForward(step, step_left); });
+// on a device handle: asynchronous, the first call runs eagerly, later calls replay one captured CUDA graph
+GX_CAPI int GXPredForward(void* handle) {
+  return Guard([&] { Handle* h = HD(handle, "GXPredForward"); if (h->dev) h->dev->Forward(); else if (h->pred) h->pred->Forward(); else h->gen->Forward(); });
 }
+GX_CAPI int GXPredPartialForward(void* handle, int step, int* step_left) {
+  return Guard([&] {
+    Handle* h = HD(handle, "GXPredPartialForward");
+    if (h->dev) h->dev->PartialForward(step, step_left); else if (h->pred) h->pred->PartialForward(step, step_left); else h->gen->PartialForward(step, step_left);
+  });
+}
+// on a device handle: waits for the handle's stream; `data` may be host or device memory
 GX_CAPI int GXPredGetOutput(void* handle, uint32_t index, float* data, uint32_t size) {
   return Guard([&] {
-    if (gxrt::capi::IsDeviceBuffer(data)) throw std::runtime_error("GXPredGetOutput: device array (the predictor writes host memory)");
-    Handle* h = H(handle); if (h->pred) h->pred->GetOutput(index, data, size); else h->gen->GetOutput(index, data, size);
+    if ((!handle || !H(handle)->dev) && gxrt::capi::IsDeviceBuffer(data))
+      throw std::runtime_error("GXPredGetOutput: device array (the predictor writes host memory)");
+    Handle* h = HD(handle, "GXPredGetOutput");
+    if (h->dev) h->dev->GetOutput(index, data, size); else if (h->pred) h->pred->GetOutput(index, data, size); else h->gen->GetOutput(index, data, size);
   });
 }
-// 1: the planned predictor (predict.h) runs this graph, 2: the general executor (train_exec.h) does
-GX_CAPI int GXPredGetEngine(void* handle, int* out) { return Guard([&] { *out = H(handle)->pred ? 1 : 2; }); }
+// 1: the planned predictor (predict.h) runs this graph on the host, 2: the general executor (train_exec.h) does, 3: the planned predictor
+// runs it on a GPU (predict_device.h)
+GX_CAPI int GXPredGetEngine(void* handle, int* out) { return Guard([&] { Handle* h = H(handle); *out = h->dev ? 3 : h->pred ? 1 : 2; }); }
 // planner statistics: bytes of the activation arena and the number of operators that run
 GX_CAPI int GXPredGetPlan(void* handle, uint64_t* arena_bytes, uint32_t* num_ops) {
   return Guard([&] {
     Handle* h = H(handle);
-    *arena_bytes = h->pred ? h->pred->ArenaBytes() : h->gen->ArenaBytes();
-    *num_ops = static_cast<uint32_t>(h->pred ? h->pred->NumOps() : h->gen->NumOps());
+    *arena_bytes = h->gen ? h->gen->ArenaBytes() : h->plan().ArenaBytes();
+    *num_ops = static_cast<uint32_t>(h->gen ? h->gen->NumOps() : h->plan().NumOps());
   });
 }
-GX_CAPI int GXPredFree(void* handle) { return Guard([&] { delete H(handle); }); }
+// a device handle waits for its stream before its memory goes back to the pool
+GX_CAPI int GXPredFree(void* handle) { return Guard([&] { delete HD(handle, "GXPredFree"); }); }
 
 GX_CAPI int GXNDListCreate(const char* nd_file_bytes, int nd_file_size, void** out, uint32_t* out_length) {
   return Guard([&] {

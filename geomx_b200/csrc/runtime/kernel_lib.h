@@ -24,6 +24,12 @@ struct Lib {
   int (*memset)(void*, int, unsigned long long, void*);
   int (*stream_sync)(void*);
   const char* (*error_string)(int);
+  int (*stream_create)(int, void**);
+  int (*stream_destroy)(void*);
+  int (*graph_begin)(void*);
+  int (*graph_end)(void*, void**);
+  int (*graph_launch)(void*, void*);
+  int (*graph_destroy)(void*);
   // device memory pool (storage_gpu.cu)
   void* (*pool_alloc)(int, uint64_t, void*);
   int (*pool_free)(int, void*, void*);
@@ -60,6 +66,12 @@ struct Lib {
   int (*softmax_bwd)(const float*, const float*, float*, long long, int, long long, int, Stream);
   int (*softmax_output_bwd)(const float*, const float*, float*, long long, int, long long, float, int, float, int, Stream);
   int (*bn_global_bwd)(const float*, const float*, const float*, const float*, const float*, float, float*, float*, float*, int, int, int, Stream);
+  // native predictor kernels (predict_ops.cu)
+  int (*map_fwd)(int, const float*, float*, long long, float, float, Stream);
+  int (*channel_affine)(const float*, float*, const float*, const float*, long long, int, long long, Stream);
+  int (*transpose)(const float*, float*, int, const long long*, const int*, Stream);
+  int (*embedding_fwd)(const float*, const float*, float*, long long, long long, long long, Stream);
+  int (*im2col_dilated)(const float*, float*, int, int, int, int, int, int, int, int, int, int, int, int, int, Stream);
 };
 
 namespace detail {
@@ -92,6 +104,12 @@ inline Lib LoadLib() {
   Resolve(h, "gx_rt_memset", &L.memset);
   Resolve(h, "gx_rt_stream_sync", &L.stream_sync);
   Resolve(h, "gx_rt_error_string", &L.error_string);
+  Resolve(h, "gx_rt_stream_create", &L.stream_create);
+  Resolve(h, "gx_rt_stream_destroy", &L.stream_destroy);
+  Resolve(h, "gx_rt_graph_begin", &L.graph_begin);
+  Resolve(h, "gx_rt_graph_end", &L.graph_end);
+  Resolve(h, "gx_rt_graph_launch", &L.graph_launch);
+  Resolve(h, "gx_rt_graph_destroy", &L.graph_destroy);
   Resolve(h, "gx_gpu_pool_alloc", &L.pool_alloc);
   Resolve(h, "gx_gpu_pool_free", &L.pool_free);
   Resolve(h, "gx_gemm_tf32", &L.gemm_tf32);
@@ -123,6 +141,11 @@ inline Lib LoadLib() {
   Resolve(h, "gx_softmax_bwd", &L.softmax_bwd);
   Resolve(h, "gx_softmax_output_bwd", &L.softmax_output_bwd);
   Resolve(h, "gx_bn_global_bwd", &L.bn_global_bwd);
+  Resolve(h, "gx_map_fwd", &L.map_fwd);
+  Resolve(h, "gx_channel_affine", &L.channel_affine);
+  Resolve(h, "gx_transpose", &L.transpose);
+  Resolve(h, "gx_embedding_fwd", &L.embedding_fwd);
+  Resolve(h, "gx_im2col_dilated", &L.im2col_dilated);
   return L;
 }
 }  // namespace detail

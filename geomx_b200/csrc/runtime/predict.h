@@ -7,7 +7,8 @@
 // that symbol.py builds structurally + the elementwise family), its own memory planner (role of src/executor/graph_executor.cc
 // InitDataEntryMemory / nnvm PlanMemory).  Both graph dialects load: this framework's `geomx_b200-symbol-1` and the reference's nnvm JSON
 // (string-valued attrs, `[node, index, version]` input triples, BatchNorm statistics as inputs 3/4), so `-symbol.json` + `.params`
-// checkpoints written by either side can be served.  GPU inference is the Python Executor's job (device tensors belong to PyTorch).
+// checkpoints written by either side can be served.  GraphPlan holds everything that does not depend on the device; Predictor runs it on
+// the host, predict_device.h::DevicePredictor runs the same plan on a GPU.
 #pragma once
 #include <algorithm>
 #include <cctype>
@@ -279,9 +280,14 @@ struct Storage {
   float* ptr = nullptr;
 };
 
-class Predictor {
+// Everything about a predictor that does not depend on where it runs: the graph (both dialects), the parameters, the input shapes, shape
+// inference, reachability and the liveness plan of the activation arena.  The host Predictor below and the device runner of
+// predict_device.h both execute this plan: order_ lists the operators that run, nodes_[i].storage names the storage each output lives in,
+// storages_ are either external (an input or a parameter) or a block of the arena at block_offset_[block] floats, and the arena holds
+// arena_floats_ floats.
+class GraphPlan {
  public:
-  Predictor(const std::string& json, const char* params, size_t param_size, const std::vector<std::string>& input_keys,
+  GraphPlan(const std::string& json, const char* params, size_t param_size, const std::vector<std::string>& input_keys,
             const std::vector<Shape>& input_shapes, const std::vector<std::string>& output_keys) {
     doc_ = std::make_shared<JValue>(JParser(json.data(), json.size()).Parse());
     BuildGraph(output_keys);
@@ -289,53 +295,33 @@ class Predictor {
     for (size_t i = 0; i < input_keys.size(); ++i) input_shapes_[input_keys[i]] = input_shapes[i];
     Plan();
   }
-  // another predictor over the same graph and parameters with its own inputs and arena (MXPredCreateMultiThread / MXPredReshape)
-  std::unique_ptr<Predictor> Clone(const std::map<std::string, Shape>* new_shapes) const {
-    std::unique_ptr<Predictor> p(new Predictor(*this));
+  // the same graph and parameters with other input shapes (those not named keep theirs), planned anew
+  void Replan(const std::map<std::string, Shape>* new_shapes) {
     if (new_shapes) for (auto& kv : *new_shapes) {
-      if (!p->input_shapes_.count(kv.first)) throw std::runtime_error("reshape: " + kv.first + " is not an input of this predictor");
-      p->input_shapes_[kv.first] = kv.second;
+      if (!input_shapes_.count(kv.first)) throw std::runtime_error("reshape: " + kv.first + " is not an input of this predictor");
+      input_shapes_[kv.first] = kv.second;
     }
-    p->Plan();
-    return p;
-  }
-
-  void SetInput(const std::string& key, const float* data, size_t size) {
-    auto it = inputs_.find(key);
-    if (it == inputs_.end()) throw std::runtime_error("SetInput: unknown input " + key);
-    if (size != it->second.size()) throw std::runtime_error("SetInput: " + key + " expects " + std::to_string(it->second.size()) + " values, got " + std::to_string(size));
-    memcpy(it->second.data(), data, size * sizeof(float));
-  }
-  void Forward() { for (size_t i = 0; i < order_.size(); ++i) Run(order_[i]); }
-  // one operator per call (MXPredPartialForward): step counts executed operators, step_left reaches 0 after the last one
-  void PartialForward(int step, int* step_left) {
-    if (step < 0 || step >= static_cast<int>(order_.size())) { *step_left = 0; return; }
-    Run(order_[step]);
-    *step_left = static_cast<int>(order_.size()) - step - 1;
+    Plan();
   }
   size_t NumOutputs() const { return heads_.size(); }
   const Shape& OutputShape(size_t i) const { return nodes_[Head(i)].shape; }
-  void GetOutput(size_t i, float* out, size_t size) const {
-    const Node& n = nodes_[Head(i)];
-    if (size != static_cast<size_t>(Numel(n.shape))) throw std::runtime_error("GetOutput: output " + std::to_string(i) + " has " + std::to_string(Numel(n.shape)) + " values, buffer holds " + std::to_string(size));
-    memcpy(out, storages_[n.storage].ptr, size * sizeof(float));
-  }
-  size_t ArenaBytes() const { return arena_.size() * sizeof(float); }
+  size_t ArenaBytes() const { return static_cast<size_t>(arena_floats_) * sizeof(float); }
   size_t NumOps() const { return order_.size(); }
 
- private:
-  Predictor(const Predictor&) = default;
+ protected:
+  GraphPlan(const GraphPlan&) = default;
   std::shared_ptr<JValue> doc_;
   std::vector<Node> nodes_;
   std::vector<Entry> heads_;
   std::shared_ptr<std::map<std::string, std::pair<Shape, std::vector<float>>>> params_;
   std::map<std::string, Shape> input_shapes_;
-  std::map<std::string, std::vector<float>> inputs_;
   std::vector<int> order_;
   std::vector<Storage> storages_;
-  std::vector<float> arena_;
+  std::vector<int64_t> block_offset_;
+  int64_t arena_floats_ = 0;
 
   int Head(size_t i) const { if (i >= heads_.size()) throw std::runtime_error("output index out of range"); return heads_[i].node; }
+  bool IsInput(const Node& nd) const { return nd.op == "null" && input_shapes_.count(nd.name) > 0; }
 
   // ---- graph construction (both dialects)
   void BuildGraph(const std::vector<std::string>& output_keys) {
@@ -388,7 +374,8 @@ class Predictor {
         heads_.push_back(Entry{found, 0});
       }
     }
-    for (auto& h : heads_) if (h.index != 0) throw std::runtime_error("secondary operator outputs cannot be predictor outputs");
+    for (auto& h : heads_)
+      if (h.index != 0) throw std::runtime_error(nodes_[h.node].name + " (" + nodes_[h.node].op + "): secondary operator outputs cannot be predictor outputs");
   }
 
   void LoadParams(const char* blob, size_t size) {
@@ -435,7 +422,7 @@ class Predictor {
     for (int i = 0; i < n; ++i) if (need[i]) for (auto& e : nodes_[i].inputs) ++consumers[e.node];
     for (auto& h : heads_) consumers[h.node] += 1 << 20;          // outputs stay alive
 
-    storages_.clear(); order_.clear(); inputs_.clear();
+    storages_.clear(); order_.clear();
     for (auto& nd : nodes_) { nd.known = false; nd.storage = -1; nd.shape.clear(); }
     std::vector<int64_t> block_size;
     std::vector<int> free_blocks;
@@ -451,11 +438,9 @@ class Predictor {
         auto in = input_shapes_.find(nd.name);
         if (in != input_shapes_.end()) {
           nd.shape = in->second; nd.known = true;
-          auto& buf = inputs_[nd.name]; buf.assign(static_cast<size_t>(Numel(nd.shape)), 0.f);
-          s.ptr = buf.data();
         } else {
           auto p = params_->find(nd.name);
-          if (p != params_->end()) { nd.shape = p->second.first; nd.known = true; s.ptr = p->second.second.data(); }
+          if (p != params_->end()) { nd.shape = p->second.first; nd.known = true; }
           // else: a label (or an unused variable) — resolved by the consumer, which must not read it
         }
         if (nd.known) for (auto d : nd.shape) if (d < 1) throw std::runtime_error(nd.name + ": empty tensors are not supported, shape " + ShapeStr(nd.shape));
@@ -493,11 +478,9 @@ class Predictor {
       order_.push_back(i);
       for (auto& e : nd.inputs) if (nodes_[e.node].storage >= 0) release(nodes_[e.node].storage);
     }
-    std::vector<int64_t> offset(block_size.size(), 0);
-    int64_t total = 0;
-    for (size_t b = 0; b < block_size.size(); ++b) { offset[b] = total; total += (block_size[b] + 15) / 16 * 16; }
-    arena_.assign(static_cast<size_t>(total), 0.f);
-    for (auto& s : storages_) if (!s.external) s.ptr = arena_.data() + offset[s.block];
+    block_offset_.assign(block_size.size(), 0);
+    arena_floats_ = 0;
+    for (size_t b = 0; b < block_size.size(); ++b) { block_offset_[b] = arena_floats_; arena_floats_ += (block_size[b] + 15) / 16 * 16; }
     for (auto& h : heads_) if (!nodes_[h.node].known) throw std::runtime_error("output " + nodes_[h.node].name + " has no shape");
   }
 
@@ -510,7 +493,6 @@ class Predictor {
     if (!s.known) throw std::runtime_error(nd.name + " (" + nd.op + "): input " + s.name + " has no value — not an input key and not in the parameter file");
     return s.shape;
   }
-  const float* InPtr(const Node& nd, size_t i) const { return storages_[In(nd, i).storage].ptr; }
   void Need(const Node& nd, size_t i, const Shape& want) const {
     if (InShape(nd, i) != want) throw std::runtime_error(nd.name + ": " + In(nd, i).name + " has shape " + ShapeStr(InShape(nd, i)) + ", expected " + ShapeStr(want));
   }
@@ -683,6 +665,61 @@ class Predictor {
     }
     nd.known = true;
   }
+};
+
+// the host runner of a GraphPlan: fp32 on the CPU, the arena and the input buffers in host memory, parameters read in place
+class Predictor : public GraphPlan {
+ public:
+  Predictor(const std::string& json, const char* params, size_t param_size, const std::vector<std::string>& input_keys,
+            const std::vector<Shape>& input_shapes, const std::vector<std::string>& output_keys)
+      : GraphPlan(json, params, param_size, input_keys, input_shapes, output_keys) {
+    Bind();
+  }
+  // another predictor over the same graph and parameters with its own inputs and arena (MXPredCreateMultiThread / MXPredReshape)
+  std::unique_ptr<Predictor> Clone(const std::map<std::string, Shape>* new_shapes) const {
+    std::unique_ptr<Predictor> p(new Predictor(*this));
+    p->Replan(new_shapes);
+    p->Bind();
+    return p;
+  }
+
+  void SetInput(const std::string& key, const float* data, size_t size) {
+    auto it = inputs_.find(key);
+    if (it == inputs_.end()) throw std::runtime_error("SetInput: unknown input " + key);
+    if (size != it->second.size()) throw std::runtime_error("SetInput: " + key + " expects " + std::to_string(it->second.size()) + " values, got " + std::to_string(size));
+    memcpy(it->second.data(), data, size * sizeof(float));
+  }
+  void Forward() { for (size_t i = 0; i < order_.size(); ++i) Run(order_[i]); }
+  // one operator per call (MXPredPartialForward): step counts executed operators, step_left reaches 0 after the last one
+  void PartialForward(int step, int* step_left) {
+    if (step < 0 || step >= static_cast<int>(order_.size())) { *step_left = 0; return; }
+    Run(order_[step]);
+    *step_left = static_cast<int>(order_.size()) - step - 1;
+  }
+  void GetOutput(size_t i, float* out, size_t size) const {
+    const Node& n = nodes_[Head(i)];
+    if (size != static_cast<size_t>(Numel(n.shape))) throw std::runtime_error("GetOutput: output " + std::to_string(i) + " has " + std::to_string(Numel(n.shape)) + " values, buffer holds " + std::to_string(size));
+    memcpy(out, storages_[n.storage].ptr, size * sizeof(float));
+  }
+
+ private:
+  Predictor(const Predictor&) = default;
+  std::map<std::string, std::vector<float>> inputs_;
+  std::vector<float> arena_;
+
+  // host memory behind the plan: zeroed input buffers, parameters in place, one arena for every other storage
+  void Bind() {
+    inputs_.clear();
+    for (auto& nd : nodes_) {
+      if (nd.op != "null" || nd.storage < 0) continue;
+      Storage& s = storages_[nd.storage];
+      if (IsInput(nd)) { auto& buf = inputs_[nd.name]; buf.assign(static_cast<size_t>(Numel(nd.shape)), 0.f); s.ptr = buf.data(); }
+      else if (nd.known) s.ptr = params_->at(nd.name).second.data();
+    }
+    arena_.assign(static_cast<size_t>(arena_floats_), 0.f);
+    for (auto& s : storages_) if (!s.external) s.ptr = arena_.data() + block_offset_[s.block];
+  }
+  const float* InPtr(const Node& nd, size_t i) const { return storages_[In(nd, i).storage].ptr; }
 
   // ---- execution
   static float Act(int kind, float v) {

@@ -12,8 +12,9 @@
  * calls on device arrays run sm_100a kernels of libgeomx_kernels.so (csrc/runtime/device_exec.h), which this library loads at the first
  * device request from its own directory — it has no link-time dependency on CUDA.  Device work is ordered on one stream per device in call
  * order; SyncCopyToCPU and the Wait* functions synchronise it.  Functions that read host bytes (Slice / At / Reshape / Detach, autograd,
- * GXKVStore*, GXPred*) refuse device arrays.  CUDA graphs, the NVLink fabric and mixed precision are driven from the Python package;
- * GXKVStore* is the TCP parameter-server plane both share.
+ * GXKVStore*, and GXPred* on host predictors) refuse device arrays.  Predictors created with dev_type 2 run on the GPU
+ * (csrc/runtime/predict_device.h) and take host or device buffers.  The NVLink fabric and mixed precision are driven from the Python
+ * package; GXKVStore* is the TCP parameter-server plane both share.
  *
  * dtype flags: 0 float32, 1 float64, 2 float16, 3 uint8, 4 int32, 5 int8, 6 int64.  grad_req: 0 null, 1 write, 3 add.
  */
@@ -237,6 +238,11 @@ int GXStorageAlloc(size_t nbytes, void** out);
 int GXStorageFree(void* p);
 
 /* ---- predict API (include/mxnet/c_predict_api.h) --------------------------------------------------------------------------------------- */
+/* dev_type 1: the host (the planned predictor, or the general executor for operators outside its set).  dev_type 2: the planned predictor
+ * on GPU dev_id with sm_100a kernels; create refuses a graph it cannot serve (the error names the node).  A device handle owns a stream,
+ * an arena and its input buffers, shares the parameters with its MultiThread / Reshape siblings, and may be driven from its own thread.
+ * SetInput copies in (host or device memory) and returns when the source has been read; Forward is asynchronous, the first one runs
+ * eagerly and every later one replays a CUDA graph; GetOutput waits and copies out (host or device memory); Free waits for the stream. */
 int GXPredCreate(const char* symbol_json, const void* param_bytes, int param_size, int dev_type, int dev_id, uint32_t num_input_nodes, const char** input_keys,
                  const uint32_t* input_shape_indptr, const uint32_t* input_shape_data, PredictorHandle* out);
 int GXPredCreatePartialOut(const char* symbol_json, const void* param_bytes, int param_size, int dev_type, int dev_id, uint32_t num_input_nodes,
@@ -253,7 +259,7 @@ int GXPredForward(PredictorHandle handle);
 int GXPredPartialForward(PredictorHandle handle, int step, int* step_left);
 int GXPredGetOutput(PredictorHandle handle, uint32_t index, float* data, uint32_t size);
 int GXPredGetPlan(PredictorHandle handle, uint64_t* arena_bytes, uint32_t* num_ops);
-int GXPredGetEngine(PredictorHandle handle, int* out);        /* 1 planned predictor, 2 general executor (operators outside the planned set) */
+int GXPredGetEngine(PredictorHandle handle, int* out);        /* 1 planned predictor, 2 general executor (operators outside the planned set), 3 planned predictor on a GPU */
 int GXPredFree(PredictorHandle handle);
 int GXNDListCreate(const char* nd_file_bytes, int nd_file_size, NDListHandle* out, uint32_t* out_length);
 int GXNDListGet(NDListHandle handle, uint32_t index, const char** out_key, const float** out_data, const uint32_t** out_shape, uint32_t* out_ndim);

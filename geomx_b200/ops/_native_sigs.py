@@ -61,6 +61,12 @@ SIGS = {
     # batchnorm.cu
     "gx_bn_fwd": [P, P, P, P, P, P, P, P, I, I, I, I, F, F, P],
     "gx_bn_bwd": [P, P, P, P, P, P, P, P, I, I, I, P],
+    # predict_ops.cu
+    "gx_map_fwd": [I, P, P, L, F, F, P],
+    "gx_channel_affine": [P, P, P, P, L, I, L, P],
+    "gx_transpose": [P, P, I, P, P, P],
+    "gx_embedding_fwd": [P, P, P, L, L, L, P],
+    "gx_im2col_dilated": [P, P] + [I] * 13 + [P],
     # hips_fabric.cu
     "gx_fabric_params_size": [],
     "gx_hips_fsa_step": [P, I, P],
