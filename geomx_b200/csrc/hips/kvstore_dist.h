@@ -106,6 +106,15 @@ class KVStoreDist {
   }
   // returns a handle for Wait()
   int Push(int key, const void* data, size_t elems, int dtype, int priority) { return PushImpl(key, data, elems, dtype, priority, true); }
+  // a float32 push of `elems` values that the caller already quantised to 2-bit words (with its own residual, e.g. on a GPU): the same
+  // message as Push sends under 2-bit compression.  The caller keeps `words` alive until the handle was waited.
+  int PushPacked2Bit(int key, const uint32_t* words, size_t elems, int priority) {
+    HIPS_CHECK_MSG(gc_.type() == CompressionType::kTwoBit, "PushPacked2Bit needs 2-bit compression");
+    const int h = Track({ZPushWords(key, words, static_cast<size_t>(GradientCompression::CompressedSize2Bit(static_cast<int64_t>(elems))), priority, nullptr)});
+    { std::lock_guard<std::mutex> lk(mu_); last_push_[key] = h; }
+    return h;
+  }
+  const GradientCompression& gradient_compression() const { return gc_; }
 
   int Pull(int key, void* out, size_t elems, int dtype, int priority) {
     // ordering: a pull of `key` observes the effect of this worker's previous push of `key` (reference: shared comm_buf_ engine var)
@@ -244,6 +253,16 @@ class KVStoreDist {
   // compressed keys live un-partitioned on their hashed server (key_codec.h CompressionPinsKey): init, push and pull agree on ONE plan
   bool Pinned(size_t elems, int dtype) const { return CompressionPinsKey(static_cast<int>(gc_.type()), elems, dtype, size_lower_bound_); }
 
+  // the 2-bit wire message of `key`: `nwords` packed words on its hashed server; `keep` holds the words alive until the send is done
+  int ZPushWords(int key, const uint32_t* words, size_t nwords, int priority, const std::function<void()>& keep) {
+    const auto& krs = Postoffice::Get()->GetServerKeyRanges(kLocal);
+    SArray<Key> keys; keys.push_back(krs[(key * 9973) % krs.size()].begin() + static_cast<Key>(key));
+    SArray<char> vals(reinterpret_cast<char*>(const_cast<uint32_t*>(words)), nwords * 4, false);
+    SArray<int> lens; lens.push_back(static_cast<int>(nwords * 4));
+    const int cmd = GetCommandType(RequestType::kCompressedPushPull, kFloat32);
+    return ps_worker_->ZPush(keys, vals, lens, cmd, keep, priority, key);
+  }
+
   int PushImpl(int key, const void* data, size_t elems, int dtype, int priority, bool allow_compress) {
     const int bytes = DTypeSize(dtype);
     std::vector<int> tss;
@@ -253,12 +272,7 @@ class KVStoreDist {
       { std::lock_guard<std::mutex> lk(mu_); res = &residual_[key]; if (res->size() != elems) res->assign(elems, 0.f); }
       auto words = std::make_shared<std::vector<uint32_t>>(GradientCompression::CompressedSize2Bit(static_cast<int64_t>(elems)));
       gc_.Quantize2Bit(static_cast<const float*>(data), res->data(), words->data(), static_cast<int64_t>(elems));
-      const auto& krs = Postoffice::Get()->GetServerKeyRanges(kLocal);
-      SArray<Key> keys; keys.push_back(krs[(key * 9973) % krs.size()].begin() + static_cast<Key>(key));
-      SArray<char> vals(reinterpret_cast<char*>(words->data()), words->size() * 4, false);
-      SArray<int> lens; lens.push_back(static_cast<int>(words->size() * 4));
-      const int cmd = GetCommandType(RequestType::kCompressedPushPull, kFloat32);
-      tss.push_back(ps_worker_->ZPush(keys, vals, lens, cmd, [words]() {}, priority, key));
+      tss.push_back(ZPushWords(key, words->data(), words->size(), priority, [words]() {}));
     } else if (enable_p3_ && allow_compress) {
       // P3: the response of the push carries the updated parameters; keep them for the following pull
       auto buf = std::make_shared<std::vector<char>>(static_cast<const char*>(data), static_cast<const char*>(data) + elems * bytes);

@@ -5,8 +5,9 @@
 // executor zeroes gradients once per Backward and fan-out accumulates, as in the host executor (train_exec.h).
 //
 // The gx_rt_* functions give the C API (compiled with g++, without CUDA headers, loading this library with dlopen) the few runtime calls it
-// needs: device count, current device, one stream per device, streams of its own (one per native predictor), copies, memset, stream
-// synchronisation and the capture / replay of a stream's work as a CUDA graph.
+// needs: device count, current device, one stream per device, streams of its own (one per native predictor), copies (peer copies
+// included), memset, stream synchronisation, stream-to-stream joins, page-locked host staging and the capture / replay of a stream's work
+// as a CUDA graph.
 #include <cuda_runtime.h>
 
 #include <mutex>
@@ -372,6 +373,42 @@ GX_API int gx_rt_graph_end(void* stream, void** out) {
 }
 GX_API int gx_rt_graph_launch(void* exec, void* stream) { return (int)cudaGraphLaunch(static_cast<cudaGraphExec_t>(exec), static_cast<cudaStream_t>(stream)); }
 GX_API int gx_rt_graph_destroy(void* exec) { return exec ? (int)cudaGraphExecDestroy(static_cast<cudaGraphExec_t>(exec)) : 0; }
+// copy between the memory of two devices (directly over NVLink / PCIe when peer access is possible, staged by the driver otherwise),
+// ordered on `stream`
+GX_API int gx_rt_memcpy_peer(void* dst, int dst_dev, const void* src, int src_dev, unsigned long long bytes, void* stream) {
+  if (bytes == 0) return 0;
+  return (int)cudaMemcpyPeerAsync(dst, dst_dev, src, src_dev, bytes, static_cast<cudaStream_t>(stream));
+}
+// makes `waiter` wait for the work queued so far on `signaller` (a stream of device signaller_dev) without blocking the host: an event of
+// the library, one per signalling stream, is recorded there and waited on.  Re-recording it later does not affect waits already enqueued.
+GX_API int gx_rt_stream_join(void* waiter, void* signaller, int signaller_dev) {
+  if (waiter == signaller) return 0;
+  static std::mutex mu;
+  static std::vector<std::pair<void*, cudaEvent_t>> events;
+  std::lock_guard<std::mutex> lk(mu);
+  cudaEvent_t ev = nullptr;
+  for (auto& e : events) if (e.first == signaller) ev = e.second;
+  int cur = 0;
+  cudaGetDevice(&cur);
+  cudaError_t e = cudaSetDevice(signaller_dev);
+  if (e == cudaSuccess && !ev) {
+    e = cudaEventCreateWithFlags(&ev, cudaEventDisableTiming);
+    if (e == cudaSuccess) events.emplace_back(signaller, ev);
+  }
+  if (e == cudaSuccess) e = cudaEventRecord(ev, static_cast<cudaStream_t>(signaller));
+  if (e == cudaSuccess) e = cudaStreamWaitEvent(static_cast<cudaStream_t>(waiter), ev, 0);
+  cudaSetDevice(cur);
+  if (e != cudaSuccess) cudaGetLastError();
+  return (int)e;
+}
+// page-locked host memory (portable: usable by every device's copies), for staging buffers whose copies must stay asynchronous
+GX_API int gx_rt_host_alloc(unsigned long long bytes, void** out) {
+  *out = nullptr;
+  const cudaError_t e = cudaHostAlloc(out, bytes ? bytes : 1, cudaHostAllocPortable);
+  if (e != cudaSuccess) { cudaGetLastError(); *out = nullptr; }
+  return (int)e;
+}
+GX_API int gx_rt_host_free(void* p) { return p ? (int)cudaFreeHost(p) : 0; }
 
 // ================================================================================================ graph operator kernels
 GX_API int gx_axpy(float* y, const float* x, float a, long long n, cudaStream_t s) {

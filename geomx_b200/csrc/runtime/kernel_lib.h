@@ -30,6 +30,10 @@ struct Lib {
   int (*graph_end)(void*, void**);
   int (*graph_launch)(void*, void*);
   int (*graph_destroy)(void*);
+  int (*memcpy_peer)(void*, int, const void*, int, unsigned long long, void*);
+  int (*stream_join)(void*, void*, int);
+  int (*host_alloc)(unsigned long long, void**);
+  int (*host_free)(void*);
   // device memory pool (storage_gpu.cu)
   void* (*pool_alloc)(int, uint64_t, void*);
   int (*pool_free)(int, void*, void*);
@@ -72,6 +76,9 @@ struct Lib {
   int (*transpose)(const float*, float*, int, const long long*, const int*, Stream);
   int (*embedding_fwd)(const float*, const float*, float*, long long, long long, long long, Stream);
   int (*im2col_dilated)(const float*, float*, int, int, int, int, int, int, int, int, int, int, int, int, int, Stream);
+  // KVStore reductions (kv_comm.cu)
+  int (*kv_sum_quantize)(float*, const float* const*, int, long long, float*, void*, float, Stream);
+  int (*kv_dequant_sum)(float*, const void* const*, int, long long, float, int, Stream);
 };
 
 namespace detail {
@@ -110,6 +117,10 @@ inline Lib LoadLib() {
   Resolve(h, "gx_rt_graph_end", &L.graph_end);
   Resolve(h, "gx_rt_graph_launch", &L.graph_launch);
   Resolve(h, "gx_rt_graph_destroy", &L.graph_destroy);
+  Resolve(h, "gx_rt_memcpy_peer", &L.memcpy_peer);
+  Resolve(h, "gx_rt_stream_join", &L.stream_join);
+  Resolve(h, "gx_rt_host_alloc", &L.host_alloc);
+  Resolve(h, "gx_rt_host_free", &L.host_free);
   Resolve(h, "gx_gpu_pool_alloc", &L.pool_alloc);
   Resolve(h, "gx_gpu_pool_free", &L.pool_free);
   Resolve(h, "gx_gemm_tf32", &L.gemm_tf32);
@@ -146,6 +157,8 @@ inline Lib LoadLib() {
   Resolve(h, "gx_transpose", &L.transpose);
   Resolve(h, "gx_embedding_fwd", &L.embedding_fwd);
   Resolve(h, "gx_im2col_dilated", &L.im2col_dilated);
+  Resolve(h, "gx_kv_sum_quantize", &L.kv_sum_quantize);
+  Resolve(h, "gx_kv_dequant_sum", &L.kv_dequant_sum);
   return L;
 }
 }  // namespace detail

@@ -12,9 +12,11 @@
  * calls on device arrays run sm_100a kernels of libgeomx_kernels.so (csrc/runtime/device_exec.h), which this library loads at the first
  * device request from its own directory — it has no link-time dependency on CUDA.  Device work is ordered on one stream per device in call
  * order; SyncCopyToCPU and the Wait* functions synchronise it.  Functions that read host bytes (Slice / At / Reshape / Detach, autograd,
- * GXKVStore*, and GXPred* on host predictors) refuse device arrays.  Predictors created with dev_type 2 run on the GPU
- * (csrc/runtime/predict_device.h) and take host or device buffers.  The NVLink fabric and mixed precision are driven from the Python
- * package; GXKVStore* is the TCP parameter-server plane both share.
+ * the raw-buffer GXKVStoreInit / Push / Pull, and GXPred* on host predictors) refuse device arrays.  Predictors created with dev_type 2 run
+ * on the GPU (csrc/runtime/predict_device.h) and take host or device buffers.  GXKVStoreInitND / PushND / PullND take host or device
+ * NDArrays on every store type: `local` reduces on the host, `device` on each key's GPU with peer copies and sm_100a kernels, and the dist
+ * stores reduce device values on the GPU before they go on the wire (csrc/runtime/kvstore_nd.h).  The NVLink fabric and mixed precision
+ * are driven from the Python package; the dist GXKVStore* types are the TCP parameter-server plane both share.
  *
  * dtype flags: 0 float32, 1 float64, 2 float16, 3 uint8, 4 int32, 5 int8, 6 int64.  grad_req: 0 null, 1 write, 3 add.
  */
@@ -173,7 +175,12 @@ int GXDataIterGetLabel(DataIterHandle h, NDArrayHandle* out);
 int GXDataIterGetIndex(DataIterHandle h, uint64_t** out_index, uint64_t* out_size);
 int GXDataIterGetPadNum(DataIterHandle h, int* pad);
 
-/* ---- KVStore (HiPS TCP plane: dist_sync / dist_async, two tiers) ----------------------------------------------------------------------- */
+/* ---- KVStore --------------------------------------------------------------------------------------------------------------------------
+ * GXKVStoreCreate types: "local", "local_update_cpu", "local_allreduce_cpu" — in-process, values reduced and kept on the host;
+ * "device", "local_allreduce_device" — in-process, each key kept and reduced on its home GPU (the device of the value given to Init);
+ * any other type (dist_sync, dist_async, ...) — a worker of the HiPS TCP parameter-server plane (two tiers).
+ * In-process stores: GetRank 0, GroupSize 1, Barrier / Wait* do nothing, SetGradientCompression("2bit") on device stores only; the raw-buffer
+ * Init / Push / Pull, the row-sparse forms and RunServer are refused (use the ND forms). */
 int GXInitPSEnv(int num, const char** keys, const char** vals);
 int GXKVStoreIsWorkerNode(int* out);
 int GXKVStoreIsServerNode(int* out);
@@ -189,6 +196,21 @@ int GXKVStorePush(KVStoreHandle h, int key, const void* data, size_t elems, int 
 int GXKVStorePull(KVStoreHandle h, int key, void* out, size_t elems, int dtype, int priority, int* handle);
 int GXKVStorePushRowSparse(KVStoreHandle h, int key, const int64_t* row_ids, size_t nrows, const float* rows, size_t row_len, int priority, int* handle);
 int GXKVStorePullRowSparse(KVStoreHandle h, int key, const int64_t* row_ids, size_t nrows, float* out, size_t row_len, int priority, int* handle);
+/* NDArray forms, host or device arrays (device arrays: float32).  Push: a key listed k times is k values, summed left to right in the
+ * order given, then stored (or handed to the updater) or sent once.  Pull: a key listed k times fills k outputs.  Init: a key may appear
+ * once and be initialised once.  The values of one key in one call are all host or all device arrays.  Local / device stores never block
+ * on device arrays: copies and sums are ordered on the devices' streams, so later work issued on any device sees the result.  Dist stores:
+ * PushND reduces device values on their GPU (and quantises them there under 2-bit compression), synchronises that GPU once and sends
+ * asynchronously; PullND requests every key of the call, waits for all replies (the keys of one call share their round trips), then
+ * enqueues the copies to the device outputs and returns. */
+int GXKVStoreInitND(KVStoreHandle h, uint32_t num, const int* keys, NDArrayHandle* vals);
+int GXKVStorePushND(KVStoreHandle h, uint32_t num, const int* keys, NDArrayHandle* vals, int priority);
+int GXKVStorePullND(KVStoreHandle h, uint32_t num, const int* keys, NDArrayHandle* vals, int priority);
+/* local / device stores: updater(key, recv, local, arg) replaces the assignment of a push; recv holds the reduced sum and local the stored
+ * value, both on the key's home (device arrays for a device key, so GXImperativeInvokeByName("sgd_update", ...) on them runs on the GPU).
+ * The handles belong to the store.  Dist stores update on their servers (command 7, or GXKVStoreRunServerEx) and refuse this call. */
+typedef void (*GXKVStoreUpdater)(int key, NDArrayHandle recv, NDArrayHandle local, void* arg);
+int GXKVStoreSetUpdater(KVStoreHandle h, GXKVStoreUpdater updater, void* arg);
 int GXKVStoreWait(KVStoreHandle h, int handle);
 int GXKVStoreWaitAll(KVStoreHandle h);
 int GXKVStoreBarrier(KVStoreHandle h);

@@ -67,6 +67,14 @@ SIGS = {
     "gx_transpose": [P, P, I, P, P, P],
     "gx_embedding_fwd": [P, P, P, L, L, L, P],
     "gx_im2col_dilated": [P, P] + [I] * 13 + [P],
+    # kv_comm.cu
+    "gx_kv_sum_quantize": [P, P, I, L, P, P, F, P],
+    "gx_kv_dequant_sum": [P, P, I, L, F, I, P],
+    # graph_ops.cu (runtime calls of the C API)
+    "gx_rt_memcpy_peer": [P, I, P, I, C.c_ulonglong, P],
+    "gx_rt_stream_join": [P, P, I],
+    "gx_rt_host_alloc": [C.c_ulonglong, P],
+    "gx_rt_host_free": [P],
     # hips_fabric.cu
     "gx_fabric_params_size": [],
     "gx_hips_fsa_step": [P, I, P],
